@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]          # this repo's CUDA path
     python bench.py --impl reference [...]                        # the reference algorithm on host cores
+    python bench.py [...] --dump-outputs DIR                      # also save the last timed step's results (.npy)
 
 Workload at N=1 = BASELINE.json configs[1]: 1M x 384 cosine (L2-normalised synthetic embeddings),
 M=16, ef_search=128, k=10, batch 10k queries.  A "step" = one batch through
@@ -57,7 +58,31 @@ def parse():
     ap.add_argument("--build-batch", type=int, default=4096, help="insert path: nodes per step (1 = sequential)")
     ap.add_argument("--build-graph-only", default="", help="(internal) build rank 0's graph, save it as .npz, exit")
     ap.add_argument("--out", default="")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the results of the last timed step as DIR/<name>.npy (float32/float64; ids -1 = none)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, arrays: dict, seed: int) -> None:
+    """Writes each array (first axis = query) as <out_dir>/<name>.npy: float32 stays float32, everything else becomes
+    float64 (exact for ids and counters below 2**53).  query_index.npy names the queries written: all of them, or a fixed
+    seeded sample when the arrays together exceed DUMP_LIMIT_BYTES."""
+    nq = len(next(iter(arrays.values())))
+    out = {"query_index": np.arange(nq, dtype=np.float64)}
+    out.update({k: v if v.dtype == np.float32 else v.astype(np.float64) for k, v in arrays.items()})
+    total = sum(v.nbytes for v in out.values())
+    if total > DUMP_LIMIT_BYTES:
+        keep = np.sort(np.random.default_rng(seed).choice(nq, nq * DUMP_LIMIT_BYTES // total, replace=False))
+        out = {k: v[keep] for k, v in out.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -209,10 +234,15 @@ def run_reference(args, rank, world):
     for it in range(args.warmup + args.steps):
         q = qb[it % qb.shape[0]][:sample]
         t = time.perf_counter()
-        g.search(q, args.k, args.ef, ob.COSINE, n_threads=cores)
+        res = g.search(q, args.k, args.ef, ob.COSINE, n_threads=cores)
         dt = time.perf_counter() - t
         if it >= args.warmup:
             times.append(dt)
+    if args.dump_outputs:
+        r_rows, r_nodes, r_dist, r_cnt, r_st = res
+        dump_outputs(args.dump_outputs, {"rows": r_rows.view(np.int64), "distances": r_dist, "counts": r_cnt,
+                                         "nodes": r_nodes.view(np.int32),
+                                         "stats": np.stack([r_st[f] for f in r_st.dtype.names], axis=1)}, args.seed)
     ms = float(np.mean(times) * 1e3)
     qps = sample / (ms / 1e3)
     line = {
@@ -299,7 +329,7 @@ def main():
     rows, dd, cnt = sharded.rows, sharded.dd, sharded.cnt  # the rank's own top-k lives inside its packed block
 
     def step(i):
-        sharded.search_batch(dq[i % nb])
+        return sharded.search_batch(dq[i % nb])
 
     def barrier():
         if world > 1:
@@ -316,16 +346,21 @@ def main():
     barrier()
     if rank == 0:
         sampler.mark()
-    idx.profile_begin(args.steps)
+    prof_steps = min(args.steps, 4096)  # the index keeps per-launch times of at most 4096 launches
+    idx.profile_begin(prof_steps)
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
     e0.record()
     for i in range(args.steps):
-        step(args.warmup + i)
+        last = step(args.warmup + i)
     e1.record()
     barrier()
     elapsed_ms = e0.elapsed_time(e1)
-    kern_ms, over_ms = idx.profile_read(args.steps)
+    kern_ms, over_ms = idx.profile_read(prof_steps)
+    if args.dump_outputs and rank == 0:  # copied now: the work below reuses these buffers
+        l_rows, l_dd, l_cnt = (t.cpu().numpy() for t in last)
+        dump_outputs(args.dump_outputs, {"rows": l_rows, "distances": l_dd, "counts": l_cnt,
+                                         "nodes": nodes.cpu().numpy(), "stats": stats.cpu().numpy()}, args.seed)
     if rank == 0 and elapsed_ms < 400:  # keep the GPU under the same load until the sampler has a few readings
         # rank-local kernel launches only: a collective here would not be matched by the other ranks
         t_end = time.time() + 0.45
@@ -348,7 +383,7 @@ def main():
         step(b)
         torch.cuda.synchronize()
         batch_bytes.append(algorithmic_bytes(stats.cpu().numpy(), args.dim, k))
-    step_bytes = [batch_bytes[(args.warmup + i) % nb] for i in range(args.steps)]
+    step_bytes = [batch_bytes[(args.warmup + i) % nb] for i in range(len(kern_ms))]
     achieved = float(np.sum(step_bytes) / (np.sum(kern_ms) / 1e3) / 1e9)
     peaks = {}
     try:

@@ -171,3 +171,22 @@ def test_bench_rank0_only_section_issues_no_collectives():
     assert "local_search(" in block
     for forbidden in ("step(", "sharded.", "dist.", "barrier("):
         assert forbidden not in block, forbidden
+
+
+def test_bench_dump_outputs_are_float_and_a_seeded_sample_when_large(tmp_path, monkeypatch):
+    import bench
+    rows = np.arange(40, dtype=np.int64).reshape(20, 2)
+    rows[3, 1] = -1
+    arrays = {"rows": rows, "distances": np.linspace(0, 1, 40, dtype=np.float32).reshape(20, 2),
+              "counts": np.full(20, 2, np.int32)}
+    bench.dump_outputs(str(tmp_path / "all"), arrays, seed=1)
+    got = {k: np.load(tmp_path / "all" / f"{k}.npy") for k in ("query_index", "rows", "distances", "counts")}
+    assert got["distances"].dtype == np.float32 and got["rows"].dtype == got["counts"].dtype == np.float64
+    assert np.array_equal(got["rows"], rows) and np.array_equal(got["query_index"], np.arange(20))
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 200)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays, seed=1)
+    qa, qb = (np.load(tmp_path / d / "query_index.npy") for d in ("a", "b"))
+    assert np.array_equal(qa, qb) and 0 < len(qa) < 20
+    assert sum(np.load(f).nbytes for f in (tmp_path / "a").iterdir()) <= 200
+    assert np.array_equal(np.load(tmp_path / "a" / "rows.npy"), rows[qa.astype(np.int64)])
