@@ -120,6 +120,28 @@ int32_t turdb_cuda_index_build(const turdb_cuda_build_params* params, uint64_t n
                                const uint64_t* row_ids, const double* random_values, int32_t device,
                                turdb_cuda_index** out);
 
+/*
+ * Appends n nodes to idx by the same insert path and parameters as turdb_cuda_index_build: the call is
+ * insert_with_callback (mod.rs:999-1084) applied to each new row in order.  New dense ids are idx.n .. idx.n + n - 1;
+ * steps continue the build's schedule from the current node count, and entry / max_level advance in id order.  On an
+ * index without an entry the first new node only becomes it (mod.rs:1020-1023).  Appending to a graph built with the
+ * same params gives the graph one build over all rows gives when the split falls on a step boundary (always with
+ * max_batch == 1).  Works on built, uploaded (index_create, hnsw_file_upload) and empty indexes.
+ *   - params->dim must equal the index dimension (TURDB_ERR_DIMENSION_MISMATCH); m, ef_construction and max_batch are
+ *     checked as by build; idx.n + n must stay below 2^31 - 1 (TURDB_ERR_UNSUPPORTED); n == 0 is a no-op.
+ *   - Device arrays grow by at least 1.5x when full, so a stream of small inserts does not copy the index every call;
+ *     turdb_cuda_index_info's device_bytes reports what is allocated.  Norms and (after enable_sq8) SQ8 rows are computed
+ *     for the new rows; the exact path's 16-bit copies are dropped and rebuilt by the next exact / SQL call.
+ *   - Failure: validation, level and slot computation, every allocation and the upload of the new rows happen before the
+ *     index changes; if any fails the index is exactly as before.  A CUDA error once the steps have started is reported
+ *     as TURDB_ERR_CUDA and leaves the index unusable: destroy it.
+ *   - Concurrency: a WRITER call.  The caller excludes every other call on the same index while it runs (the reference's
+ *     RwLock write guard); search calls on an index are re-entrant among themselves, not with insert.  The device is
+ *     synchronised before replaced buffers are freed, so work enqueued earlier on any stream finishes first.
+ */
+int32_t turdb_cuda_index_insert(turdb_cuda_index* idx, const turdb_cuda_build_params* params, uint64_t n,
+                                const float* vectors, const uint64_t* row_ids, const double* random_values);
+
 /* The index's graph as flat host arrays (the turdb_cuda_graph layout; counts = valid ids per row); every pointer is
  * nullable.  up_adj / up_cnt hold *n_up_slots rows (call once with only n_up_slots to size them). */
 int32_t turdb_cuda_index_export_graph(turdb_cuda_index* idx, float* vectors, uint64_t* row_ids, uint8_t* levels,

@@ -65,6 +65,12 @@ struct turdb_cuda_index {
   uint32_t* d_up_adj = nullptr;
   uint64_t* d_row_ids = nullptr;
   uint8_t* d_levels = nullptr;
+  // per-list state the insert path's link kernels append to (graph_insert.inl): valid entries of each level-0 / upper
+  // list and the node owning each upper slot; kept for the index's lifetime so that later inserts can back-link
+  uint8_t* d_l0_cnt = nullptr;
+  uint8_t* d_up_cnt = nullptr;
+  uint32_t* d_up_owner = nullptr;
+  uint64_t cap_n = 0, cap_slots = 0;       // allocated nodes / upper slots of every per-node / per-slot array (>= n, n_up_slots)
   void* d_row_map = nullptr;               // device copy of the arena's gather4 tensor map (TURDB_GATHER4 builds)
   uint32_t g4_boxw = 0;
   uint8_t* d_arena_sq8 = nullptr;          // SQ8 rows: dim codes | pad | min | scale, sq8_row_bytes apart (enable_sq8)
@@ -109,8 +115,8 @@ struct DeviceGuard {
 // One warp per adjacency row: entries >= count become INVALID, ids are range-checked, and a repeated id
 // keeps only its first occurrence (the reference's visited set skips the repeats, search.rs:338, so the
 // traversal is unchanged; the kernel's lock-free visited table relies on rows without repeats).  The row is
-// re-packed to a prefix in stored order.
-__global__ void sanitize_adj_kernel(uint32_t* adj, const uint8_t* cnt, uint64_t rows, uint32_t width,
+// re-packed to a prefix in stored order, and cnt[r] becomes the number of ids it keeps.
+__global__ void sanitize_adj_kernel(uint32_t* adj, uint8_t* cnt, uint64_t rows, uint32_t width,
                                     uint64_t n, uint32_t* bad) {
   const uint64_t r = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const uint32_t lane = threadIdx.x & 31;
@@ -130,6 +136,15 @@ __global__ void sanitize_adj_kernel(uint32_t* adj, const uint8_t* cnt, uint64_t 
   if (lane < width) adj[r * width + lane] = kInvalid;
   __syncwarp();
   if (keep) adj[r * width + __popc(km & ((1u << lane) - 1))] = v;
+  if (lane == 0) cnt[r] = (uint8_t)__popc(km);
+}
+
+// up_owner[up_base[i] + l] = i for l < levels[i] (slots no node claims keep what they held)
+__global__ void up_owner_kernel(const uint8_t* levels, const uint32_t* up_base, uint64_t n, uint32_t first,
+                                uint32_t* up_owner) {
+  const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  for (uint32_t l = 0; l < levels[i]; ++l) up_owner[(size_t)up_base[i] + l] = first + (uint32_t)i;
 }
 
 // dot(b, b) per arena row in the reference's AVX2 lane order (cosine_avx2's norm_b chain)
@@ -212,6 +227,9 @@ int32_t turdb_cuda_index_destroy(turdb_cuda_index* idx) {
     cudaFree(idx->d_up_adj);
     cudaFree(idx->d_row_ids);
     cudaFree(idx->d_levels);
+    cudaFree(idx->d_l0_cnt);
+    cudaFree(idx->d_up_cnt);
+    cudaFree(idx->d_up_owner);
     cudaFree(idx->d_row_map);
     cudaFree(idx->d_arena_sq8);
     cudaFree(idx->d_norm2_sq8);
@@ -330,27 +348,29 @@ int32_t turdb_cuda_index_create(const turdb_cuda_graph* g, int32_t device, turdb
     const uint64_t slots = g->n_up_slots;
     IDX_TRY(cudaMalloc(&idx->d_up_adj, std::max<uint64_t>(slots, 1) * kUp * 4));
     if (slots) IDX_TRY(cudaMemcpy(idx->d_up_adj, g->up_adj, slots * kUp * 4, cudaMemcpyHostToDevice));
-    idx->device_bytes = arena_bytes + n * 4 + n * kL0 * 4 + n * 4 + n * 8 + n + slots * kUp * 4;
+    IDX_TRY(cudaMalloc(&idx->d_l0_cnt, n));
+    IDX_TRY(cudaMalloc(&idx->d_up_cnt, std::max<uint64_t>(slots, 1)));
+    IDX_TRY(cudaMalloc(&idx->d_up_owner, std::max<uint64_t>(slots, 1) * 4));
+    idx->device_bytes = arena_bytes + n * 4 + n * kL0 * 4 + n * 4 + n * 8 + n + slots * kUp * 4 + n + slots * 5;
     idx->n_up_slots = slots;
+    idx->cap_n = n;
+    idx->cap_slots = slots;
 
-    // counts -> INVALID padding, id range check
-    uint8_t* d_cnt = nullptr;
+    // counts -> INVALID padding, id range check; the counts kept are those of the sanitised rows
     uint32_t* d_bad = nullptr;
-    IDX_TRY(cudaMalloc(&d_cnt, std::max<uint64_t>(n, slots)));
     IDX_TRY(cudaMalloc(&d_bad, 4));
     IDX_TRY(cudaMemset(d_bad, 0, 4));
-    IDX_TRY(cudaMemcpy(d_cnt, g->l0_cnt, n, cudaMemcpyHostToDevice));
-    {
-      sanitize_adj_kernel<<<(unsigned)((n * 32 + 255) / 256), 256>>>(idx->d_l0_adj, d_cnt, n, kL0, n, d_bad);
-    }
+    IDX_TRY(cudaMemcpy(idx->d_l0_cnt, g->l0_cnt, n, cudaMemcpyHostToDevice));
+    sanitize_adj_kernel<<<(unsigned)((n * 32 + 255) / 256), 256>>>(idx->d_l0_adj, idx->d_l0_cnt, n, kL0, n, d_bad);
     if (slots) {
-      IDX_TRY(cudaMemcpy(d_cnt, g->up_cnt, slots, cudaMemcpyHostToDevice));
-      sanitize_adj_kernel<<<(unsigned)((slots * 32 + 255) / 256), 256>>>(idx->d_up_adj, d_cnt, slots, kUp, n, d_bad);
+      IDX_TRY(cudaMemcpy(idx->d_up_cnt, g->up_cnt, slots, cudaMemcpyHostToDevice));
+      sanitize_adj_kernel<<<(unsigned)((slots * 32 + 255) / 256), 256>>>(idx->d_up_adj, idx->d_up_cnt, slots, kUp, n, d_bad);
+      IDX_TRY(cudaMemset(idx->d_up_owner, 0xFF, slots * 4));
+      up_owner_kernel<<<(unsigned)((n + 255) / 256), 256>>>(idx->d_levels, idx->d_up_base, n, 0, idx->d_up_owner);
     }
     norm2_kernel<<<(unsigned)((n * 4 + 255) / 256), 256>>>(idx->d_arena, dim, ds, n, idx->d_norm2);
     uint32_t bad = 0;
     IDX_TRY(cudaMemcpy(&bad, d_bad, 4, cudaMemcpyDeviceToHost));
-    cudaFree(d_cnt);
     cudaFree(d_bad);
     IDX_TRY(cudaGetLastError());
     if (bad) {
@@ -379,13 +399,14 @@ int32_t turdb_cuda_index_enable_sq8(turdb_cuda_index* idx, uint8_t* out_rows, ui
   const uint32_t dim = idx->ix.dim;
   const uint32_t row_bytes = (((dim + 3) & ~3u) + 8 + 15) & ~15u;
   if (!idx->d_arena_sq8 && n) {
-    CUDA_TRY(cudaMalloc(&idx->d_arena_sq8, n * row_bytes));
-    CUDA_TRY(cudaMalloc(&idx->d_norm2_sq8, n * 4));
+    const uint64_t cap = idx->cap_n;  // sized like the arena: turdb_cuda_index_insert encodes appended rows in place
+    CUDA_TRY(cudaMalloc(&idx->d_arena_sq8, cap * row_bytes));
+    CUDA_TRY(cudaMalloc(&idx->d_norm2_sq8, cap * 4));
     sq8_encode_kernel<<<(unsigned)((n * 32 + 255) / 256), 256>>>(idx->d_arena, dim, idx->ix.ds, n, idx->d_arena_sq8, row_bytes);
     sq8_norm2_kernel<<<(unsigned)((n * 4 + 255) / 256), 256>>>(idx->d_arena_sq8, dim, row_bytes, n, idx->d_norm2_sq8);
     CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaDeviceSynchronize());
-    idx->device_bytes += n * row_bytes + n * 4;
+    idx->device_bytes += cap * row_bytes + cap * 4;
   }
   idx->sq8_row_bytes = row_bytes;
   if (out_row_bytes) *out_row_bytes = row_bytes;

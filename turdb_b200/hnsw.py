@@ -77,12 +77,14 @@ def _ptr(a, t):
 class CudaHnswIndex:
     """A flattened HNSW graph resident on one B200 (device arena + fixed-stride adjacency)."""
 
-    def __init__(self, handle, dim: int, n: int, metric: DistanceFunction, device: int):
+    def __init__(self, handle, dim: int, n: int, metric: DistanceFunction, device: int, build_params=None):
         self._h = handle
         self.dim = dim
         self.n = n
         self._metric = DistanceFunction(metric)
         self.device = device
+        # (m, ef_construction, mode) that `insert` uses when its arguments are omitted; None: they must be given
+        self._build_params = build_params
 
     # ---- construction -------------------------------------------------------------------
     @classmethod
@@ -134,7 +136,42 @@ class CudaHnswIndex:
         h = C.c_void_p()
         _check(_lib.load().turdb_cuda_index_build(C.byref(bp), n, _ptr(vec, C.c_float), _ptr(rid, C.c_uint64),
                                                   _ptr(rnd, C.c_double), device, C.byref(h)))
-        return cls(h, dim, n, metric, device)
+        return cls(h, dim, n, metric, device, build_params=(m, ef_construction, mode))
+
+    def insert(self, vectors, row_ids, random_values, m: int | None = None, ef_construction: int | None = None,
+               mode: int | None = None, max_batch: int = 4096):
+        """Append rows by the insert path (turdb_cuda_index_insert): PersistentHnswIndex::insert_with_callback for each
+        row in order, new node ids self.n .. self.n + len - 1.  row_ids and random_values (the (0, 1] draw select_level
+        uses) come from the caller, as in the reference's DML hook.  m / ef_construction / mode default to those of
+        `build` (or of the `.hnsw` header for HnswFile.upload, mode 1).  A writer call: no other call may use this index
+        while it runs.  Raises ValueError before touching the device on bad shapes, dtypes or parameters."""
+        vec = np.asarray(vectors)
+        if vec.dtype.kind != "f" or vec.ndim != 2 or vec.shape[1] != self.dim:
+            raise ValueError(f"vectors must be float [n, {self.dim}], got {vec.dtype} {vec.shape}")
+        n = vec.shape[0]
+        if row_ids is None or random_values is None:
+            raise ValueError("row_ids and random_values are required (one per inserted row)")
+        rid = np.asarray(row_ids)
+        rnd = np.asarray(random_values)
+        if rid.dtype.kind not in "ui" or rid.shape != (n,):
+            raise ValueError(f"row_ids must be integer [{n}], got {rid.dtype} {rid.shape}")
+        if rid.dtype.kind == "i" and n and rid.min() < 0:
+            raise ValueError("row_ids must be non-negative")
+        if rnd.dtype.kind != "f" or rnd.shape != (n,):
+            raise ValueError(f"random_values must be float [{n}], got {rnd.dtype} {rnd.shape}")
+        if None in (m, ef_construction, mode):
+            if self._build_params is None:
+                raise ValueError("m, ef_construction and mode are required: this index was not built or read from a file")
+            bm, bef, bmode = self._build_params
+            m, ef_construction, mode = (bm if m is None else m, bef if ef_construction is None else ef_construction,
+                                        bmode if mode is None else mode)
+        vec = np.ascontiguousarray(vec, dtype=np.float32)
+        rid = np.ascontiguousarray(rid, dtype=np.uint64)
+        rnd = np.ascontiguousarray(rnd, dtype=np.float64)
+        bp = _lib.BuildParams(self.dim, int(m), int(ef_construction), int(mode), int(max_batch), 0)
+        _check(_lib.load().turdb_cuda_index_insert(self._h, C.byref(bp), n, _ptr(vec, C.c_float), _ptr(rid, C.c_uint64),
+                                                   _ptr(rnd, C.c_double)))
+        self.n += n
 
     def export_graph(self, with_vectors: bool = True) -> dict:
         """The graph the device holds, as the flat arrays from_graph takes (turdb_cuda_index_export_graph)."""

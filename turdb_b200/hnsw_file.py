@@ -133,4 +133,4 @@ class HnswFile:
         h = C.c_void_p()
         _check(L.turdb_cuda_hnsw_file_upload(self._h, vec_p, pres_p, cb, None, device, C.byref(h)))
         m = self.distance_fn() if metric is None else DistanceFunction(metric)
-        return CudaHnswIndex(h, dim, self.n_total, m, device)
+        return CudaHnswIndex(h, dim, self.n_total, m, device, build_params=(self.info["m"], self.info["ef_construction"], 1))
