@@ -297,6 +297,33 @@ int32_t turdb_cuda_sql_topk_batch_device(turdb_cuda_index* idx, const float* d_q
                                          uint32_t* d_out_counts, void* stream);
 
 /*
+ * ---- the SQL distance-range scan: WHERE vec <op> '[...]' <cmp> radius LIMIT limit OFFSET offset, batched ---------
+ * Replaces a Filter over a full scan when the predicate is Column <op> literal <cmp> constant: one call = nq
+ * statements against the same table, statement q with literal queries[q] and constant radius[q] (f64).  op: 0 `<->`,
+ * 1 `<=>`, 2 `<#>` — the projected value of src/sql/predicate.rs:1634-1688 (f32, sequential: sqrt L2, 1 - cos with
+ * NULL on a zero norm, +dot), widened to f64.  cmp: 0 `<`, 1 `<=`, 2 `>`, 3 `>=`.  Only the near direction is
+ * supported (`<`/`<=` with `<->` and `<=>`, `>`/`>=` with `<#>`); any other pair is TURDB_ERR_UNSUPPORTED.
+ *
+ * Row i qualifies iff its value compares true against radius[q] in f64; a NULL value and an absent vector (a +inf row)
+ * never do.  out_counts[q] = the number of qualifying rows; rows [offset, offset + limit) of them, in scan order
+ * (= dense node id order), are written to out_row_ids [nq][limit] and their values to out_vals (nullable); unused
+ * slots are TURDB_INVALID_ROW / NaN.  limit = 0 is a COUNT (out_row_ids may then be NULL).
+ *
+ * The certified tensor-core filter of the exact path runs one pass with a per-statement threshold derived from the
+ * radius (widened by its score-error bound and a bound on the f32 evaluation error of the value), so no qualifying row
+ * is dropped; its survivors are decided by the exact value.  A statement with more survivors than the candidate buffer
+ * holds (DESIGN §4.6) is redone by a kernel that runs the reference's loop over every row.  Dimension limits as for
+ * turdb_cuda_sql_topk_batch.
+ */
+int32_t turdb_cuda_sql_range_batch(turdb_cuda_index* idx, const float* queries, uint32_t query_dim, uint32_t nq,
+                                   uint8_t op, uint8_t cmp, const double* radius, uint32_t limit, uint32_t offset,
+                                   uint64_t* out_row_ids, double* out_vals, uint32_t* out_counts);
+int32_t turdb_cuda_sql_range_batch_device(turdb_cuda_index* idx, const float* d_queries, uint32_t query_dim,
+                                          uint32_t nq, uint8_t op, uint8_t cmp, const double* d_radius,
+                                          uint32_t limit, uint32_t offset, uint64_t* d_out_row_ids,
+                                          double* d_out_vals, uint32_t* d_out_counts, void* stream);
+
+/*
  * ---- multi-GPU: merge of per-shard top-k after the all-gather (one sub-index per GPU) --------
  * gathered_* are [n_shards][nq][k] device arrays (the NCCL all-gather output); ties order by
  * (distance, row_id).  Output [nq][k].

@@ -16,7 +16,7 @@ for _m, _mn in ((0, "l2"), (1, "cosine"), (2, "ip")):
     UNITS.append(("search_kernels_staged.cu", [f"TURDB_TU_METRIC={_m}"], f"search_staged_{_mn}.o"))
     UNITS.append(("search_kernels_direct.cu", [f"TURDB_TU_METRIC={_m}"], f"search_direct_{_mn}.o"))
 DEPS = ["turdb_cuda.cu", "common.cuh", "hnsw_search.cuh", "search_kernels.h", "search_kernels_staged.cu", "search_kernels_direct.cu",
-        "exact_search.cuh", "exact_abi.inl", "gather_probe.cuh", "hnsw_file.inl", "sql_topk.inl", "graph_insert.inl",
+        "exact_search.cuh", "exact_abi.inl", "gather_probe.cuh", "hnsw_file.inl", "sql_topk.inl", "sql_range.inl", "graph_insert.inl",
         os.path.join("..", "..", "include", "turdb_cuda.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-Wall"]

@@ -222,6 +222,64 @@ __global__ void query_slack_kernel(const float* __restrict__ queries, uint32_t d
   }
 }
 
+// Fixed threshold of the range form (turdb_cuda_sql_range_batch, DESIGN §4.6): per statement, a filter key below which no
+// row can satisfy `v <cmp> radius[q]`, v = the f32 projected value (sql_projection).  Only the near direction exists
+// (v <= r for L2 / cosine, v >= r for IP), and `<` is treated as `<=` (a superset).  In f64, rounded toward admitting:
+//   e  = slack[q] / 2 = 1.01 e(q) >= |filter key - real key|                  (query_slack_kernel)
+//   g  = gamma_n = n u / (1 - n u), u = 2^-24: the bound of a sequential f32 sum of n rounded products, relative to
+//        the sum of the absolute products
+//   L2 : v = fl(sqrt(fl(sum fl(fl(q_i - x_i)^2)))) >= |q - x| (1 - u) sqrt(1 - gamma_{n+2}), so v <= r implies
+//        |q - x| <= R = r / ((1 - u) sqrt(1 - gamma_{n+2})) and the key q.x - |x|^2/2 = (|q|^2 - |q - x|^2) / 2
+//        >= (|q|^2 - R^2) / 2;                                         tau = (|q|^2 - R^2) / 2 - e
+//   cos: the three f32 sums, two sqrts, product, quotient and 1 - . give |v - (1 - cos)| <= Ec (below), so v <= r
+//        implies cos >= 1 - r - Ec; the key is |q| cos up to the rows' f32 scaling by rsqrtf(norm2) (relative
+//        g + 4u, norm2 is itself an f32 sum);                          tau = |q| (1 - r - Ec) - |q| (g + 4u) - e
+//   IP : |v - q.x| <= g |q| max|x|, max|x| <= Xn + Dx (arena_max2);   tau = r - g |q| (Xn + Dx) - e
+// and every tau is lowered by 2^-30 of its terms' magnitudes (the f64 arithmetic here) and rounded down to f32.  A NaN
+// radius compares false for every row (tau = +inf), a zero query under cosine is NULL for every row (+inf), and a
+// bound that is not finite (a query overflowing the FP16 copy, an arena with +inf rows) admits every row (tau = -inf).
+__global__ void range_thresh_kernel(const float* __restrict__ queries, uint32_t dim, uint32_t nq, int metric,
+                                    const double* __restrict__ radius, const float* __restrict__ slack,
+                                    const uint32_t* __restrict__ arena_max2, float* __restrict__ thresh) {
+  const uint32_t q = blockIdx.x * blockDim.x + threadIdx.x;
+  if (q >= nq) return;
+  double qq = 0.0;  // |q|^2: every product is exact in f64, the sum is off by at most dim 2^-53 of it
+  for (uint32_t i = 0; i < dim; ++i) {
+    const double v = (double)queries[(size_t)q * dim + i];
+    qq = fma(v, v, qq);
+  }
+  const double u = 0x1p-24, r = radius[q], e = 0.5 * (double)slack[q], qn = sqrt(qq);
+  const double g = dim * u / (1.0 - dim * u);
+  double t, mag;
+  if (r != r) {
+    t = INFINITY;
+    mag = 0.0;
+  } else if (metric == kL2) {
+    const double g2 = (dim + 2) * u / (1.0 - (dim + 2) * u);
+    const double R = fmax(r, 0.0) / ((1.0 - u) * sqrt(1.0 - g2));
+    t = 0.5 * (qq - R * R) - e;
+    mag = qq + R * R + e;
+  } else if (metric == kCosine) {
+    if (qq == 0.0) {
+      t = INFINITY;
+      mag = 0.0;
+    } else {
+      const double a = g + u;                                   // |n1 / |x| - 1|, |n2 / |q| - 1|
+      const double B = (1.0 + a) * (1.0 + a) * (1.0 + u) - 1.0;  // |fl(n1 n2) / (|x||q|) - 1|
+      const double Ec = ((u + B) + g * (1.0 + u)) / (1.0 - B) + 3.0 * u;
+      t = qn * (1.0 - r - Ec) - qn * (g + 4.0 * u) - e;
+      mag = qn * (1.0 + fabs(r) + Ec) + e;
+    }
+  } else {
+    const double X = (double)__uint_as_float(arena_max2[0]) + (double)__uint_as_float(arena_max2[1]);
+    t = r - g * qn * X - e;
+    mag = fabs(r) + g * qn * X + e;
+  }
+  t -= 0x1p-30 * mag;
+  if (t != t) t = -INFINITY;
+  thresh[q] = __double2float_rd(t);
+}
+
 // Ranking key of a score for column (vector) j, larger = closer (the query's own norm does not change ranks) — in every
 // case what the contraction itself produces:  L2: q.x - |x|^2/2 (three augmented columns of the L2 copy, to_half_kernel)
 // cosine: q.x on rows pre-scaled by 1/|x|      IP: q.x

@@ -1055,5 +1055,6 @@ extern "C" int32_t turdb_cuda_index_gather_probe(turdb_cuda_index* idx, uint32_t
   return TURDB_OK;
 }
 #include "sql_topk.inl"
+#include "sql_range.inl"
 #include "hnsw_file.inl"
 #include "graph_insert.inl"

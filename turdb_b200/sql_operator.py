@@ -8,6 +8,9 @@ Host-side mirror of the reference's TopK executor for that statement shape (kahf
 A planner replaces TopKExec(scan) by this operator when order_by[0] is `Column <op> literal`
 (src/sql/ast.rs:907-909); many statements over one table go through ONE launch (`VectorScanBatch`,
 BASELINE.json config 5's batch path).  All arithmetic is below the C ABI (csrc/sql_topk.inl).
+
+The distance-range scan `SELECT ... WHERE vec <op> '[...]' <cmp> r [LIMIT k [OFFSET o]]` (a Filter over the scan) runs
+through `VectorRangeScanBatch` (csrc/sql_range.inl).
 """
 from __future__ import annotations
 
@@ -72,6 +75,73 @@ class VectorScanBatch:
                                                             int(self.op), int(self.project or 0), 1 if self.use_index else 0,
                                                             self.ef_search, d_rows, d_keys, d_proj or None, d_counts,
                                                             stream or None))
+
+
+class RangeCmp(enum.IntEnum):
+    Lt = 0   # `<`
+    Le = 1   # `<=`
+    Gt = 2   # `>`
+    Ge = 3   # `>=`
+
+
+def range_direction_supported(op: VectorOp, cmp: RangeCmp) -> bool:
+    """The near direction only: `<->` / `<=>` below a radius, `<#>` above a threshold."""
+    return (VectorOp(op) == VectorOp.InnerProduct) == (RangeCmp(cmp) in (RangeCmp.Gt, RangeCmp.Ge))
+
+
+class VectorRangeScanBatch:
+    """nq statements `SELECT ... FROM t WHERE vec <op> literal_i <cmp> radius_i LIMIT limit OFFSET offset` against one
+    table (csrc/sql_range.inl).  A row qualifies iff its projected f32 value (predicate.rs:1634-1688), widened to f64,
+    compares true against radius_i; NULL values and absent vectors never do.  Rows come back in scan (primary-key)
+    order; limit = 0 is a COUNT.  Raises ValueError before the library is called on a bad op / cmp pair, shape or dtype."""
+
+    def __init__(self, index: CudaHnswIndex, op: VectorOp, cmp: RangeCmp, limit: int, offset: int = 0):
+        try:
+            self.op, self.cmp = VectorOp(op), RangeCmp(cmp)
+        except ValueError as e:
+            raise ValueError(f"unknown operator: {e}") from None
+        if not range_direction_supported(self.op, self.cmp):
+            raise ValueError(f"{self.op.name} {self.cmp.name}: only the near direction is supported "
+                             "(<-> and <=> with < or <=, <#> with > or >=)")
+        limit, offset = int(limit), int(offset)
+        if not (0 <= limit < 2**32 and 0 <= offset < 2**32):
+            raise ValueError("limit and offset must be in [0, 2^32)")
+        self.index, self.limit, self.offset = index, limit, offset
+
+    def _inputs(self, literals, radius):
+        q = np.asarray(literals)
+        if q.ndim == 1:
+            q = q[None, :]
+        if q.dtype.kind != "f" or q.ndim != 2 or q.shape[1] != self.index.dim:
+            raise ValueError(f"literals must be float [nq, {self.index.dim}], got {q.dtype} {q.shape}")
+        r = np.asarray(radius)
+        if r.ndim == 0:
+            r = r[None]
+        if r.dtype.kind not in "fiu" or r.shape != (q.shape[0],):
+            raise ValueError(f"radius must be one number per statement [{q.shape[0]}], got {r.dtype} {r.shape}")
+        return np.ascontiguousarray(q, dtype=np.float32), np.ascontiguousarray(r, dtype=np.float64)
+
+    def execute(self, literals, radius) -> tuple[np.ndarray, np.ndarray, np.ndarray]:
+        """-> (row_ids u64 [nq, limit], values f64 [nq, limit], counts u32 [nq] = ALL qualifying rows); unused slots are
+        INVALID_ROW / NaN."""
+        q, r = self._inputs(literals, radius)
+        nq = q.shape[0]
+        lim = max(self.limit, 1)
+        rows = np.full((nq, lim), INVALID_ROW, np.uint64)
+        vals = np.full((nq, lim), np.nan, np.float64)
+        counts = np.zeros(nq, np.uint32)
+        _check(_lib.load().turdb_cuda_sql_range_batch(self.index._h, _ptr(q, C.c_float), q.shape[1], nq, int(self.op),
+                                                      int(self.cmp), _ptr(r, C.c_double), self.limit, self.offset,
+                                                      _ptr(rows, C.c_uint64), _ptr(vals, C.c_double), _ptr(counts, C.c_uint32)))
+        return rows[:, :self.limit], vals[:, :self.limit], counts
+
+    def execute_device(self, d_literals: int, nq: int, d_radius: int, d_rows: int, d_counts: int, stream: int = 0,
+                       d_vals: int = 0):
+        """Device-resident form: raw device addresses (literals f32 [nq][dim], radius f64 [nq], rows u64 [nq][limit],
+        counts u32 [nq], values f64 [nq][limit] or 0), enqueued on `stream` (no host synchronisation)."""
+        _check(_lib.load().turdb_cuda_sql_range_batch_device(self.index._h, d_literals, self.index.dim, nq, int(self.op),
+                                                             int(self.cmp), d_radius, self.limit, self.offset,
+                                                             d_rows or None, d_vals or None, d_counts, stream or None))
 
 
 class VectorTopKExec:
