@@ -324,6 +324,33 @@ int32_t turdb_cuda_sql_range_batch_device(turdb_cuda_index* idx, const float* d_
                                           double* d_out_vals, uint32_t* d_out_counts, void* stream);
 
 /*
+ * ---- the nearest rows within a radius: WHERE vec <where_op> '[...]' <cmp> radius ORDER BY vec <order_op> '[...]'
+ *      LIMIT limit OFFSET offset, batched (both clauses with the same literal) ------------------------------------------
+ * The reference plans TopK(Filter(Scan)): its heap sees the rows that pass the Filter, in primary-key order.  One call =
+ * nq such statements against the same table, statement q with literal queries[q] and constant radius[q] (f64).
+ *   Filter: exactly turdb_cuda_sql_range_batch's predicate (where_op 0 `<->`, 1 `<=>`, 2 `<#>`; cmp 0 `<`, 1 `<=`,
+ *           2 `>`, 3 `>=`; near direction only, other pairs TURDB_ERR_UNSUPPORTED; NULL values and absent vectors never
+ *           qualify).
+ *   TopK:   exactly turdb_cuda_sql_topk_batch's result over the qualifying rows, row for row, order among equal keys
+ *           included: order_op 0 `<->` or 1 `<=>` (`<#>` is TURDB_ERR_UNSUPPORTED), f64 keys, out_row_ids / out_keys
+ *           [nq][limit], out_proj (nullable) the value of `SELECT vec <proj_op> '[...]'`, out_counts[q] = rows returned,
+ *           unused slots TURDB_INVALID_ROW / NaN, limit + offset <= TURDB_SQL_MAX_LIMIT_PLUS_OFFSET.  Order among NULL
+ *           keys (e.g. WHERE `<->`, ORDER BY `<=>` on a zero-norm row) is unspecified.
+ * Operators and limit + offset are checked before the index.  The range scan's single filter pass finds the candidates;
+ * each statement's survivors go through the exact predicate in scan order and the replayed heap.  A statement with
+ * more survivors than the candidate buffer holds is redone by the reference's loop over every row (DESIGN §4.6).
+ */
+int32_t turdb_cuda_sql_range_topk_batch(turdb_cuda_index* idx, const float* queries, uint32_t query_dim, uint32_t nq,
+                                        uint8_t where_op, uint8_t cmp, const double* radius, uint8_t order_op,
+                                        uint8_t proj_op, uint32_t limit, uint32_t offset, uint64_t* out_row_ids,
+                                        double* out_keys, double* out_proj, uint32_t* out_counts);
+int32_t turdb_cuda_sql_range_topk_batch_device(turdb_cuda_index* idx, const float* d_queries, uint32_t query_dim,
+                                               uint32_t nq, uint8_t where_op, uint8_t cmp, const double* d_radius,
+                                               uint8_t order_op, uint8_t proj_op, uint32_t limit, uint32_t offset,
+                                               uint64_t* d_out_row_ids, double* d_out_keys, double* d_out_proj,
+                                               uint32_t* d_out_counts, void* stream);
+
+/*
  * ---- multi-GPU: merge of per-shard top-k after the all-gather (one sub-index per GPU) --------
  * gathered_* are [n_shards][nq][k] device arrays (the NCCL all-gather output); ties order by
  * (distance, row_id).  Output [nq][k].

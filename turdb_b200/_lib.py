@@ -55,7 +55,8 @@ EXPORTS = [
     "turdb_cuda_hnsw_file_upload", "turdb_cuda_sql_topk_batch", "turdb_cuda_sql_topk_batch_device",
     "turdb_cuda_index_enable_sq8", "turdb_cuda_search_batch_sq8_device", "turdb_cuda_shards_search_batch",
     "turdb_cuda_index_build", "turdb_cuda_index_export_graph", "turdb_cuda_index_insert",
-    "turdb_cuda_sql_range_batch", "turdb_cuda_sql_range_batch_device",
+    "turdb_cuda_sql_range_batch", "turdb_cuda_sql_range_batch_device", "turdb_cuda_sql_range_topk_batch",
+    "turdb_cuda_sql_range_topk_batch_device",
 ]
 
 _lib = None
@@ -98,6 +99,9 @@ def load():
     L.turdb_cuda_sql_range_batch.argtypes = [vp, pf, u32, u32, u8, u8, C.POINTER(C.c_double), u32, u32, pu64,
                                              C.POINTER(C.c_double), pu32]
     L.turdb_cuda_sql_range_batch_device.argtypes = [vp, vp, u32, u32, u8, u8, vp, u32, u32, vp, vp, vp, vp]
+    L.turdb_cuda_sql_range_topk_batch.argtypes = [vp, pf, u32, u32, u8, u8, C.POINTER(C.c_double), u8, u8, u32, u32, pu64,
+                                                  C.POINTER(C.c_double), C.POINTER(C.c_double), pu32]
+    L.turdb_cuda_sql_range_topk_batch_device.argtypes = [vp, vp, u32, u32, u8, u8, vp, u8, u8, u32, u32, vp, vp, vp, vp, vp]
     L.turdb_cuda_index_enable_sq8.argtypes = [vp, pu8, u64, pu32]
     L.turdb_cuda_search_batch_sq8_device.argtypes = [vp, vp, u32, u32, u32, u32, u8, vp, vp, vp, vp, vp, vp, vp]
     L.turdb_cuda_shards_search_batch.argtypes = [C.POINTER(vp), u32, pf, u32, u32, u32, u32, u8, pu64, pf, pu32]

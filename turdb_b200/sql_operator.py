@@ -10,7 +10,8 @@ A planner replaces TopKExec(scan) by this operator when order_by[0] is `Column <
 BASELINE.json config 5's batch path).  All arithmetic is below the C ABI (csrc/sql_topk.inl).
 
 The distance-range scan `SELECT ... WHERE vec <op> '[...]' <cmp> r [LIMIT k [OFFSET o]]` (a Filter over the scan) runs
-through `VectorRangeScanBatch` (csrc/sql_range.inl).
+through `VectorRangeScanBatch` (csrc/sql_range.inl), and both clauses together with one literal,
+`... WHERE vec <op> '[...]' < r ORDER BY vec <op> '[...]' LIMIT k` (TopK over the Filter), through `VectorRangeTopKBatch`.
 """
 from __future__ import annotations
 
@@ -142,6 +143,63 @@ class VectorRangeScanBatch:
         _check(_lib.load().turdb_cuda_sql_range_batch_device(self.index._h, d_literals, self.index.dim, nq, int(self.op),
                                                              int(self.cmp), d_radius, self.limit, self.offset,
                                                              d_rows or None, d_vals or None, d_counts, stream or None))
+
+
+SQL_MAX_LIMIT_PLUS_OFFSET = 512  # TURDB_SQL_MAX_LIMIT_PLUS_OFFSET, include/turdb_cuda.h
+
+
+class VectorRangeTopKBatch:
+    """nq statements `SELECT [vec <project> literal_i] ... FROM t WHERE vec <where_op> literal_i <cmp> radius_i
+    ORDER BY vec <order_op> literal_i LIMIT limit OFFSET offset` against one table (csrc/sql_range.inl): the reference's
+    TopK over exactly the rows its Filter lets through, row for row — VectorRangeScanBatch's predicate, VectorScanBatch's
+    keys and heap order.  Raises ValueError before the library is called on an unknown or unsupported operator (the far
+    direction, `<#>` as the sort key), limit + offset > SQL_MAX_LIMIT_PLUS_OFFSET, or a bad literal / radius."""
+
+    def __init__(self, index: CudaHnswIndex, where_op: VectorOp, cmp: RangeCmp, order_op: VectorOp, limit: int,
+                 offset: int = 0, project: VectorOp | None = None):
+        self._where = VectorRangeScanBatch(index, where_op, cmp, limit, offset)  # operator pair, window and input checks
+        try:
+            self.order_op = VectorOp(order_op)
+            self.project = None if project is None else VectorOp(project)
+        except ValueError as e:
+            raise ValueError(f"unknown operator: {e}") from None
+        if self.order_op == VectorOp.InnerProduct:
+            raise ValueError("ORDER BY <#> is NULL for every row in the reference; only <-> and <=> are sort keys")
+        w = self._where
+        if w.limit + w.offset > SQL_MAX_LIMIT_PLUS_OFFSET:
+            raise ValueError(f"limit + offset = {w.limit + w.offset} > {SQL_MAX_LIMIT_PLUS_OFFSET}")
+        self.index, self.where_op, self.cmp, self.limit, self.offset = index, w.op, w.cmp, w.limit, w.offset
+        self.projected = None
+
+    def execute(self, literals, radius) -> tuple[np.ndarray, np.ndarray, np.ndarray]:
+        """-> (row_ids u64 [nq, limit], keys f64 [nq, limit] (NaN = NULL), counts u32 [nq] = rows returned); unused slots
+        are INVALID_ROW / NaN.  The projected values, when asked for, are left in `self.projected` (f64 [nq, limit])."""
+        q, r = self._where._inputs(literals, radius)
+        nq = q.shape[0]
+        lim = max(self.limit, 1)
+        rows = np.full((nq, lim), INVALID_ROW, np.uint64)
+        keys = np.full((nq, lim), np.nan, np.float64)
+        proj = np.full((nq, lim), np.nan, np.float64) if self.project is not None else None
+        counts = np.zeros(nq, np.uint32)
+        _check(_lib.load().turdb_cuda_sql_range_topk_batch(self.index._h, _ptr(q, C.c_float), q.shape[1], nq,
+                                                           int(self.where_op), int(self.cmp), _ptr(r, C.c_double),
+                                                           int(self.order_op), int(self.project or 0), self.limit,
+                                                           self.offset, _ptr(rows, C.c_uint64), _ptr(keys, C.c_double),
+                                                           _ptr(proj, C.c_double) if proj is not None else None,
+                                                           _ptr(counts, C.c_uint32)))
+        self.projected = None if proj is None else proj[:, :self.limit]
+        return rows[:, :self.limit], keys[:, :self.limit], counts
+
+    def execute_device(self, d_literals: int, nq: int, d_radius: int, d_rows: int, d_keys: int, d_counts: int,
+                       stream: int = 0, d_proj: int = 0):
+        """Device-resident form: raw device addresses (literals f32 [nq][dim], radius f64 [nq], rows u64 [nq][limit],
+        keys f64 [nq][limit], counts u32 [nq], projected values f64 [nq][limit] or 0), enqueued on `stream` (no host
+        synchronisation)."""
+        _check(_lib.load().turdb_cuda_sql_range_topk_batch_device(self.index._h, d_literals, self.index.dim, nq,
+                                                                  int(self.where_op), int(self.cmp), d_radius,
+                                                                  int(self.order_op), int(self.project or 0), self.limit,
+                                                                  self.offset, d_rows or None, d_keys or None,
+                                                                  d_proj or None, d_counts, stream or None))
 
 
 class VectorTopKExec:
