@@ -142,6 +142,28 @@ int32_t turdb_cuda_index_build(const turdb_cuda_build_params* params, uint64_t n
 int32_t turdb_cuda_index_insert(turdb_cuda_index* idx, const turdb_cuda_build_params* params, uint64_t n,
                                 const float* vectors, const uint64_t* row_ids, const double* random_values);
 
+/*
+ * Deletes nodes from idx: node_ids[0 .. n) (host array of dense node ids, the ids the visibility bitmap uses) become rows
+ * the table no longer holds.  Node ids, rows and graph links stay as they are (no compaction, no repair).
+ *   - Deleting a deleted node does nothing; duplicates are allowed; n == 0 only reports the count.  *out_n_deleted
+ *     (nullable) receives the number of deleted nodes in the index after the call.
+ *   - An id >= idx.n, or node_ids null with n > 0, is TURDB_ERR_INVALID_ARGUMENT, checked before anything changes.  The
+ *     first delete allocates a bitmap of one bit per node capacity; if that fails (TURDB_ERR_OUT_OF_MEMORY) the index
+ *     is unchanged.
+ *   - Every read path treats a deleted row as absent from the table.  Traversals (search_batch[_device],
+ *     search_batch_sq8_device, shards_search_batch) are search_filtered (search.rs:352-398) with visibility `live`, or
+ *     `visible AND live` when the caller passes a bitmap: deleted nodes are traversed, never returned.  sql_topk_batch,
+ *     sql_range_batch, sql_range_topk_batch and bruteforce_topk return what the same call returns on an index holding
+ *     only the live rows (row ids, keys, values and counts; bruteforce's node ids stay this index's ids); sql_topk's
+ *     use_index form is TopK over the rows the filtered traversal returns.
+ *   - turdb_cuda_index_insert ignores deletions (the reference's insert path reads no visibility): deleted nodes stay
+ *     waypoints and may receive back-links; appended rows are live.  hnsw_file_upload tombstones and export_graph are
+ *     unaffected.  An index without a delete runs exactly the launches it ran before this call existed.
+ *   - Concurrency: a WRITER call, like insert.  Work enqueued earlier on any stream answers as before the call (the
+ *     device is synchronised before bits change in place).
+ */
+int32_t turdb_cuda_index_delete(turdb_cuda_index* idx, uint64_t n, const uint32_t* node_ids, uint64_t* out_n_deleted);
+
 /* The index's graph as flat host arrays (the turdb_cuda_graph layout; counts = valid ids per row); every pointer is
  * nullable.  up_adj / up_cnt hold *n_up_slots rows (call once with only n_up_slots to size them). */
 int32_t turdb_cuda_index_export_graph(turdb_cuda_index* idx, float* vectors, uint64_t* row_ids, uint8_t* levels,

@@ -28,7 +28,14 @@ struct DeviceIndex {
   uint32_t ds;
   uint32_t entry;
   uint32_t max_level;
+  // rows still in the table (turdb_cuda_index_delete): bit i of word i / 64; null until the first delete = every row.
+  // The traversal never reads it (the launch hands it over as the visibility bitmap); the exact / SQL kernels do.
+  const uint64_t* live;
 };
+
+__device__ __forceinline__ bool node_live(const DeviceIndex& ix, uint32_t id) {
+  return !ix.live || ((ix.live[id >> 6] >> (id & 63)) & 1ull) != 0;
+}
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
   return static_cast<uint32_t>(__cvta_generic_to_shared(p));

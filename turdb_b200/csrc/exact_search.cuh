@@ -879,7 +879,8 @@ __global__ void __launch_bounds__(32 * kThreshWarps) exact_threshold_kernel(uint
                                                                             uint32_t* cand_cnt, uint32_t* cand_id, float* cand_key,
                                                                             float* thresh, const float* __restrict__ slack,
                                                                             uint32_t* kept, uint32_t* qflags, uint32_t* arch_cnt,
-                                                                            uint32_t* arch_id, uint32_t arch_cap) {
+                                                                            uint32_t* arch_id, uint32_t arch_cap,
+                                                                            const uint64_t* __restrict__ live) {
   __shared__ uint32_t hist[kThreshWarps][256];
   const uint32_t w = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t q = blockIdx.x * kThreshWarps + w;
@@ -892,16 +893,32 @@ __global__ void __launch_bounds__(32 * kThreshWarps) exact_threshold_kernel(uint
   bool flag = raw_cnt > cap;
   float* keys = cand_key + (size_t)q * cap;
   uint32_t* ids = cand_id + (size_t)q * cap;
+  // deleted rows (live bit clear; live == null: none) are dropped here, so nothing downstream sees them: they are
+  // neither archived nor kept, and tau is the kprime-th best LIVE key
+  auto is_live = [&](uint32_t id) { return !live || ((live[id >> 6] >> (id & 63)) & 1ull) != 0; };
   if (arch_id) {
-    const uint32_t base = arch_cnt[q], n_new = cnt - prev;
-    for (uint32_t i = lane; i < n_new; i += 32)
-      if (base + i < arch_cap) arch_id[(size_t)q * arch_cap + base + i] = ids[prev + i];
+    const uint32_t base = arch_cnt[q];
+    uint32_t n_new = 0;
+    for (uint32_t b = prev; b < cnt; b += 32) {
+      const uint32_t i = b + lane;
+      const uint32_t id = i < cnt ? ids[i] : 0u;
+      const bool ok = i < cnt && is_live(id);
+      const uint32_t bal = __ballot_sync(kFullMask, ok);
+      const uint32_t pos = base + n_new + __popc(bal & lt_mask);
+      if (ok && pos < arch_cap) arch_id[(size_t)q * arch_cap + pos] = id;
+      n_new += __popc(bal);
+    }
     __syncwarp();
     if (lane == 0) arch_cnt[q] = min(base + n_new, arch_cap);
     if (base + n_new > arch_cap) flag = true;
   }
+  uint32_t n_live = cnt;
+  if (live) {
+    n_live = 0;
+    for (uint32_t b = 0; b < cnt; b += 32) n_live += __popc(__ballot_sync(kFullMask, b + lane < cnt && is_live(ids[b + lane])));
+  }
   float tau = -INFINITY;
-  if (kprime > 0 && cnt >= kprime) {
+  if (kprime > 0 && n_live >= kprime) {
     uint32_t prefix = 0, remaining = kprime;  // the remaining-th largest among the keys whose high digits equal prefix
     for (int shift = 24; shift >= 0; shift -= 8) {
       for (uint32_t i = lane; i < 256; i += 32) h[i] = 0;
@@ -913,7 +930,7 @@ __global__ void __launch_bounds__(32 * kThreshWarps) exact_threshold_kernel(uint
         uint32_t u = 0;
         if (ok) {
           u = key_to_ordered(keys[i]);
-          ok = (u & hi_mask) == prefix;
+          ok = (u & hi_mask) == prefix && is_live(ids[i]);
         }
         const uint32_t digit = (u >> shift) & 255u;
         const uint32_t active = __ballot_sync(kFullMask, ok);
@@ -967,7 +984,7 @@ __global__ void __launch_bounds__(32 * kThreshWarps) exact_threshold_kernel(uint
     if (i < cnt) {
       kf = keys[i];
       id = ids[i];
-      ok = kf >= tau;
+      ok = kf >= tau && is_live(id);
     }
     const uint32_t bal = __ballot_sync(kFullMask, ok);
     __syncwarp();  // every lane has read its entry before any lane overwrites one (targets are <= own index)
@@ -1101,10 +1118,11 @@ __global__ void __launch_bounds__(256) exact_stream_topk_kernel(DeviceIndex ix, 
       __syncthreads();
       if (warp == 0) {
         const uint32_t cnt = (uint32_t)min((uint64_t)64, (uint64_t)(ix.n - base));
+        const uint64_t lw = ix.live ? ix.live[base >> 6] : ~0ull;  // the chunk is one word of the live bitmap
         for (uint32_t half = 0; half < cnt; half += 32) {
           const uint32_t j = half + lane;
           const float dj = j < cnt ? cd[j] : INFINITY;
-          uint32_t mask = __ballot_sync(kFullMask, j < cnt && (len < k || dj < ld[k - 1]));
+          uint32_t mask = __ballot_sync(kFullMask, j < cnt && ((lw >> j) & 1ull) && (len < k || dj < ld[k - 1]));
           while (mask) {
             const uint32_t l = __ffs(mask) - 1;
             mask &= mask - 1;

@@ -84,6 +84,9 @@ struct turdb_cuda_index {
   float l2_scale = 1.f;                    // power of two the L2 copy's bias columns are divided by (the query side carries it)
   uint32_t* d_bf16_max2 = nullptr;         // [3 copies][2]: max |v - bf16(v)|_2, max |bf16(v)|_2 over rows (float bits); [6]: max
                                            // |value|; [7]: max |x|^2
+  uint64_t* d_live = nullptr;              // turdb_cuda_index_delete: one bit per node, (cap_n + 63) / 64 words; null until the
+                                           // first delete (ix.live points to it)
+  uint64_t n_deleted = 0;                  // nodes in [0, n) whose live bit is clear
   cudaMemPool_t pool = nullptr;            // per-index stream-ordered scratch pool (never trimmed)
   uint64_t device_bytes = 0;
   uint64_t n_up_slots = 0;
@@ -198,6 +201,29 @@ __global__ void sq8_norm2_kernel(const uint8_t* rows, uint32_t dim, uint32_t row
   if (quad < n && (threadIdx.x & 3) == 0) out[quad] = r;
 }
 
+// live bitmap (turdb_cuda_index_delete): bits [lo, hi) set, one thread per word
+__global__ void live_set_kernel(uint64_t* live, uint64_t lo, uint64_t hi) {
+  const uint64_t w = lo / 64 + (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (w * 64 >= hi) return;
+  const uint64_t a = max(lo, w * 64), b = min(hi, w * 64 + 64);
+  const uint64_t run = b - a == 64 ? ~0ull : (1ull << (b - a)) - 1ull;
+  live[w] |= run << (a - w * 64);
+}
+
+// clears the bits of ids[0, n); *cleared counts the bits that were set (a repeated id clears nothing the second time)
+__global__ void live_clear_kernel(uint64_t* live, const uint32_t* __restrict__ ids, uint64_t n, unsigned long long* cleared) {
+  const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const uint32_t id = ids[i];
+  const unsigned long long bit = 1ull << (id & 63);
+  if (atomicAnd(reinterpret_cast<unsigned long long*>(live) + (id >> 6), ~bit) & bit) atomicAdd(cleared, 1ull);
+}
+
+__global__ void live_and_kernel(const uint64_t* __restrict__ a, const uint64_t* __restrict__ b, uint64_t words, uint64_t* out) {
+  const uint64_t w = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (w < words) out[w] = a[w] & b[w];
+}
+
 extern "C" {
 
 uint32_t turdb_cuda_abi_version(void) { return TURDB_CUDA_ABI_VERSION; }
@@ -237,6 +263,7 @@ int32_t turdb_cuda_index_destroy(turdb_cuda_index* idx) {
     cudaFree(idx->d_arena_bf16n);
     cudaFree(idx->d_arena_bf16l2);
     cudaFree(idx->d_bf16_max2);
+    cudaFree(idx->d_live);
     for (cudaEvent_t ev : idx->prof_events) cudaEventDestroy(ev);
     cudaFree(idx->d_dbg);
     cudaFree(idx->d_tstats);
@@ -425,6 +452,62 @@ int32_t turdb_cuda_index_info(const turdb_cuda_index* idx, uint64_t* n, uint32_t
   if (max_level) *max_level = idx->ix.max_level;
   if (entry) *entry = idx->ix.entry;
   if (device_bytes) *device_bytes = idx->device_bytes;
+  return TURDB_OK;
+}
+
+// Deletion is state of the index: the live bitmap, allocated by the first delete at the node capacity (insert keeps it
+// in step), every node of [0, n) set, then the deleted bits cleared.  Node ids, rows and graph stay as they are.
+int32_t turdb_cuda_index_delete(turdb_cuda_index* idx, uint64_t n, const uint32_t* node_ids, uint64_t* out_n_deleted) {
+  if (n && !node_ids) return fail(TURDB_ERR_INVALID_ARGUMENT, "node_ids is null");
+  if (!idx) return fail(TURDB_ERR_INVALID_ARGUMENT, "idx is null");
+  const uint64_t n_nodes = idx->ix.n;
+  for (uint64_t i = 0; i < n; ++i)
+    if (node_ids[i] >= n_nodes)
+      return fail(TURDB_ERR_INVALID_ARGUMENT, "node_ids[%llu] = %u >= n = %llu", (unsigned long long)i, node_ids[i],
+                  (unsigned long long)n_nodes);
+  if (n) {
+    DeviceGuard guard(idx->device);
+    if (!guard.ok) return fail(TURDB_ERR_CUDA, "cudaSetDevice(%d) failed", idx->device);
+    const uint64_t words = (idx->cap_n + 63) / 64;
+    uint64_t* fresh = nullptr;
+    if (!idx->d_live) CUDA_TRY(cudaMalloc(&fresh, words * 8));
+    else CUDA_TRY(cudaDeviceSynchronize());  // the bits change in place: work enqueued earlier, on any stream, reads them first
+    uint64_t* live = fresh ? fresh : idx->d_live;
+    cudaStream_t stream = nullptr;
+    uint8_t* scr = nullptr;  // ids | cleared count
+    const size_t off_cnt = (n * 4 + 15) & ~(size_t)15;
+    unsigned long long cleared = 0;
+    cudaError_t e = cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking);
+    if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&scr, off_cnt + 8, idx->pool, stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(scr, node_ids, n * 4, cudaMemcpyHostToDevice, stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(scr + off_cnt, 0, 8, stream);
+    if (e == cudaSuccess && fresh) {
+      e = cudaMemsetAsync(fresh, 0, words * 8, stream);
+      live_set_kernel<<<(unsigned)((n_nodes + 64 * 256 - 1) / (64 * 256)), 256, 0, stream>>>(fresh, 0, n_nodes);
+    }
+    if (e == cudaSuccess) {
+      live_clear_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(live, (const uint32_t*)scr, n,
+                                                                         (unsigned long long*)(scr + off_cnt));
+      e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) e = cudaMemcpyAsync(&cleared, scr + off_cnt, 8, cudaMemcpyDeviceToHost, stream);
+    if (scr) cudaFreeAsync(scr, stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(stream);
+    if (stream) cudaStreamDestroy(stream);
+    if (e != cudaSuccess) {
+      cudaFree(fresh);
+      return fail(e == cudaErrorMemoryAllocation ? TURDB_ERR_OUT_OF_MEMORY : TURDB_ERR_CUDA, "delete failed: %s",
+                  cudaGetErrorString(e));
+    }
+    std::lock_guard<std::mutex> lk(idx->mu);
+    if (fresh) {
+      idx->d_live = fresh;
+      idx->ix.live = fresh;
+      idx->device_bytes += words * 8;
+    }
+    idx->n_deleted += cleared;
+  }
+  if (out_n_deleted) *out_n_deleted = idx->n_deleted;
   return TURDB_OK;
 }
 
@@ -674,7 +757,10 @@ static int32_t search_batch_device_impl(turdb_cuda_index* idx, const float* d_qu
   }
   const uint32_t budget = (uint32_t)idx->max_smem_optin;
   const uint64_t nn = idx->ix.n;
-  const bool filt = d_visible != nullptr;
+  // deleted rows (turdb_cuda_index_delete) are rows the table no longer holds: search_filtered over `live`, or over
+  // `visible AND live` (combined below, in pool scratch).  The insert path's searches read no visibility.
+  const uint64_t* d_live = ins ? nullptr : idx->ix.live;
+  const bool filt = d_visible != nullptr || d_live != nullptr;
   // form: short FP32 rows -> one warp per query, registers as the landing zone; long rows -> team + TMA staging
   // (measured, r02: 2M x 128 clustered, 4 new rows per hop: direct 2.64 ms, staged 3.00; 1M x 128 SIFT-like, 24 new rows
   // per hop: direct 7.9 ms, staged 4.9) — so the direct form needs short rows AND few of them per hop; until a launch
@@ -790,7 +876,9 @@ static int32_t search_batch_device_impl(turdb_cuda_index* idx, const float* d_qu
   uint2* d_fovf = nullptr;
   uint32_t* d_gv = nullptr;
   uint2* d_fovf_fb = nullptr;
+  uint64_t* d_vis_live = nullptr;
   auto release = [&]() {
+    if (d_vis_live) cudaFreeAsync(d_vis_live, stream);
     if (d_fovf_fb) cudaFreeAsync(d_fovf_fb, stream);
     if (d_gv) cudaFreeAsync(d_gv, stream);
     if (d_fovf) cudaFreeAsync(d_fovf, stream);
@@ -801,6 +889,14 @@ static int32_t search_batch_device_impl(turdb_cuda_index* idx, const float* d_qu
   if (e == cudaSuccess && filt) e = cudaMallocFromPoolAsync(&d_fovf, (size_t)grid * f_ocap_main * sizeof(uint2), idx->pool, stream);
   if (e == cudaSuccess) e = cudaMallocFromPoolAsync(&d_gv, (size_t)fb_ctas * vis_words * 4, idx->pool, stream);
   if (e == cudaSuccess && filt) e = cudaMallocFromPoolAsync(&d_fovf_fb, (size_t)fb_ctas * f_ocap_fb * sizeof(uint2), idx->pool, stream);
+  if (e == cudaSuccess && d_live && d_visible) {
+    const uint64_t words = (nn + 63) / 64;
+    e = cudaMallocFromPoolAsync(&d_vis_live, words * 8, idx->pool, stream);
+    if (e == cudaSuccess) {
+      live_and_kernel<<<(unsigned)((words + 255) / 256), 256, 0, stream>>>(d_visible, d_live, words, d_vis_live);
+      e = cudaGetLastError();
+    }
+  }
   if (e != cudaSuccess) {
     release();
     return fail(e == cudaErrorMemoryAllocation ? TURDB_ERR_OUT_OF_MEMORY : TURDB_ERR_CUDA, "traversal scratch: %s", cudaGetErrorString(e));
@@ -824,7 +920,7 @@ static int32_t search_batch_device_impl(turdb_cuda_index* idx, const float* d_qu
   a.global_visited = nullptr;
   a.vis_words = 0;
   a.dbg = idx->d_dbg;
-  a.visible = d_visible;
+  a.visible = d_vis_live ? d_vis_live : (d_visible ? d_visible : d_live);
   a.row_map = lay.g4_pieces ? idx->d_row_map : nullptr;
   a.rows = sq8 ? idx->d_arena_sq8 : reinterpret_cast<const uint8_t*>(idx->d_arena);
   a.row_bytes = lay.vec_bytes;

@@ -173,6 +173,23 @@ class CudaHnswIndex:
                                                    _ptr(rnd, C.c_double)))
         self.n += n
 
+    def delete(self, node_ids) -> int:
+        """Delete rows by dense node id (turdb_cuda_index_delete) and return how many nodes of the index are deleted
+        after the call.  Every read path then treats them as rows the table no longer holds; node ids and the graph stay
+        as they are.  Deleting a deleted node, duplicates and an empty list are allowed.  A writer call, like insert.
+        Raises ValueError before touching the device on a non-integer dtype, a shape other than [n] or an id outside
+        [0, node_count())."""
+        ids = np.asarray(node_ids)
+        if ids.ndim != 1 or (ids.size and ids.dtype.kind not in "ui"):
+            raise ValueError(f"node_ids must be integer [n], got {ids.dtype} {ids.shape}")
+        if ids.size and (int(ids.min()) < 0 or int(ids.max()) >= self.n):
+            raise ValueError(f"node_ids must lie in [0, {self.n}), got [{int(ids.min())}, {int(ids.max())}]")
+        ids = np.ascontiguousarray(ids, dtype=np.uint32)
+        out = C.c_uint64(0)
+        _check(_lib.load().turdb_cuda_index_delete(self._h, ids.size, _ptr(ids, C.c_uint32) if ids.size else None,
+                                                   C.byref(out)))
+        return int(out.value)
+
     def export_graph(self, with_vectors: bool = True) -> dict:
         """The graph the device holds, as the flat arrays from_graph takes (turdb_cuda_index_export_graph)."""
         L = _lib.load()
