@@ -269,7 +269,7 @@ int32_t turdb_cuda_index_gather_probe(turdb_cuda_index* idx, uint32_t ctas_per_s
  * The filter kernel has a one-CTA (tcgen05 cta_group::1) and a two-CTA (cta_group::2, clusters of 2) form; the library
  * picks by dimension (two-CTA above 64 dims, one-CTA when no cluster fits).  Results do not depend on the form.
  * Measurement switches (environment, read per call; never needed in production): TURDB_EXACT_PAIR=0/1 forces a form,
- * TURDB_EXACT_GROWTH=g sets the slice growth factor, TURDB_EXACT_TILE_N=128 runs 128-vector tiles over four accumulators, TURDB_EXACT_FORCE_BF16=1 (read when an index's 16-bit copy is built) forbids FP16 operands,
+ * TURDB_EXACT_GROWTH=g sets the slice growth factor, TURDB_EXACT_FORCE_BF16=1 (read when an index's 16-bit copy is built) forbids FP16 operands,
  * TURDB_EXACT_VERBOSE=1 prints the chosen form to stderr; TURDB_EXACT_SLACK_SCALE and TURDB_EXACT_DIAG make the filter
  * UNCERTIFIED / wrong on purpose and exist only to time its parts.
  */

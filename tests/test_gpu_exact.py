@@ -53,12 +53,11 @@ def test_exact_topk_matches_reference(gpu_required, n, dim, nq, k):
 
 
 @pytest.mark.parametrize("env", [{"TURDB_EXACT_PAIR": "0"}, {"TURDB_EXACT_PAIR": "1"}, {"TURDB_EXACT_GROWTH": "2"},
-                                 {"TURDB_EXACT_PAIR": "0", "TURDB_EXACT_GROWTH": "7"}, {"TURDB_EXACT_TILE_N": "128"},
-                                 {"TURDB_EXACT_TILE_N": "256"}, {"TURDB_EXACT_TILE_N": "128", "TURDB_EXACT_PAIR": "0"}])
+                                 {"TURDB_EXACT_PAIR": "0", "TURDB_EXACT_GROWTH": "7"}])
 def test_every_form_of_the_filter_gives_the_same_answer(gpu_required, monkeypatch, env):
-    """One-CTA (cta_group::1) and two-CTA (cta_group::2) kernels, 256-vector tiles over two accumulators or 128-vector tiles over
-    four, other slice growths: switches the library reads per call.  The answer must not depend on any of them — ids and distance
-    bits equal to the default configuration's and to the reference's exact top-k."""
+    """One-CTA (cta_group::1) and two-CTA (cta_group::2) kernels, other slice growths: switches the library reads per call.
+    The answer must not depend on any of them — ids and distance bits equal to the default configuration's and to the
+    reference's exact top-k."""
     n, nq, k = 6000, 300, 10  # 300 queries: a second (partly empty) query block in both forms
     for dim in (96, 384):
         x = ds.gaussian_latent(n, dim, seed=dim, normalise=False)

@@ -79,42 +79,9 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t
       : "memory");
 }
 
-// TMA tile::gather4 (sm_100): FOUR rows of a 2-D tensor (box {W, 1} in its tensor map), columns [c0, c0 + W), land
-// back to back in shared memory (row j at dst + j * W * elem) with one instruction; rows beyond the tensor read as
-// zeros and move no data.  Probed on B200 (tools/micro/gather4_probe.cu): box {W, 4} is an illegal instruction.
-__device__ __forceinline__ void tma_gather4(uint32_t dst, const void* map, int32_t c0, int32_t r0, int32_t r1, int32_t r2,
-                                            int32_t r3, uint32_t bar) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cta.global.tile::gather4.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4, %5, %6}], [%7];" ::"r"(dst),
-      "l"(map), "r"(c0), "r"(r0), "r"(r1), "r"(r2), "r"(r3), "r"(bar)
-      : "memory");
-}
-__device__ __forceinline__ void tma_gather4_prefetch(const void* map, int32_t c0, int32_t r0, int32_t r1, int32_t r2, int32_t r3) {
-  asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global.tile::gather4 [%0, {%1, %2, %3, %4, %5}];" ::"l"(map), "r"(c0),
-               "r"(r0), "r"(r1), "r"(r2), "r"(r3)
-               : "memory");
-}
-
 // L2 prefetch of a byte range (cp.async.bulk.prefetch.L2; 16 B aligned, size % 16 == 0): no destination, no barrier.
 __device__ __forceinline__ void bulk_prefetch_l2(const void* src, uint32_t bytes) {
   asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(src), "r"(bytes) : "memory");
-}
-
-// ---- per-thread 16 B async copies (cp.async; SASS: LDGSTS) ---------------------------------------
-// 32 lanes x 16 B = 512 contiguous bytes per warp instruction, no uniform-register operands (a bulk copy
-// costs ~10 instructions per issuing lane because its operands must be moved to uniform registers).
-__device__ __forceinline__ void cp_async16(uint32_t dst, const void* src) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-// wait until at most `n` of this thread's committed groups are pending (n in 0..3)
-__device__ __forceinline__ void cp_async_wait_pending(uint32_t n) {
-  switch (n) {
-    case 0: asm volatile("cp.async.wait_group 0;" ::: "memory"); break;
-    case 1: asm volatile("cp.async.wait_group 1;" ::: "memory"); break;
-    case 2: asm volatile("cp.async.wait_group 2;" ::: "memory"); break;
-    default: asm volatile("cp.async.wait_group 3;" ::: "memory"); break;
-  }
 }
 
 // ---- the reference's AVX2 reduction order, one QUAD (4 lanes) per vector ---------------------

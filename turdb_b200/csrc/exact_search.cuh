@@ -373,14 +373,11 @@ __device__ __forceinline__ void tmem_ld_32x32b_x32_nowait(uint32_t taddr, uint32
 // Barriers: TMA of both CTAs completes on the LEADER's full barriers (.cta_group::2 form, leader arms 2x the bytes);
 // tcgen05.commit multicasts "stage free" / "accumulator full" to both CTAs; both CTAs' epilogue warps arrive remotely on
 // the leader's "accumulator drained" barrier.
-#ifndef TURDB_EXACT_TILE_N
-#define TURDB_EXACT_TILE_N 256
-#endif
 #ifndef TURDB_EXACT_EPI_COLS
 #define TURDB_EXACT_EPI_COLS 64
 #endif
 constexpr uint32_t kTileM = 128;   // queries per CTA tile (UMMA M per CTA)
-constexpr uint32_t kTileN = TURDB_EXACT_TILE_N;   // vectors per MMA tile (UMMA N): 128 or 256
+constexpr uint32_t kTileN = 256;   // vectors per MMA tile (UMMA N)
 constexpr uint32_t kChunkK = 64;   // 16-bit elements per 128 B swizzle row
 constexpr uint32_t kChunkBytes = kTileM * kChunkK * 2;   // 16 KB per A (query) chunk
 constexpr uint32_t kMaxStages = 8; // B pipeline depth is chosen at launch (as many stages as fit)
@@ -389,14 +386,13 @@ constexpr uint32_t kEpiWarps = 4 * (kTileN / kEpiCols);  // one per (TMEM lane q
 constexpr uint32_t kEpiThreads = 32 * kEpiWarps;
 constexpr uint32_t kExactThreads = 64 + kEpiThreads;  // warp 0 TMA, warp 1 MMA + TMEM alloc, then the epilogue warps
 constexpr uint32_t kWq = 64;       // entries of a warp's candidate queue (flushed when more than 32 are pending)
-static_assert(kTileN == 128 || kTileN == 256, "UMMA N");
 static_assert(kEpiCols == 32 || kEpiCols == 64 || kEpiCols == 128, "epilogue slice");
 static_assert(kExactThreads <= 1024, "CTA size");
 
 // bytes of one B (vector) chunk a CTA stages: the whole tile's rows, or half of them in the two-CTA form
-__host__ __device__ constexpr uint32_t exact_b_chunk_bytes(bool pair, uint32_t tile_n) { return (pair ? tile_n / 2 : tile_n) * kChunkK * 2; }
-__host__ __device__ constexpr uint32_t exact_stage_bytes(bool stream_a, bool pair, uint32_t tile_n) {
-  return (stream_a ? kChunkBytes : 0u) + exact_b_chunk_bytes(pair, tile_n);
+__host__ __device__ constexpr uint32_t exact_b_chunk_bytes(bool pair) { return (pair ? kTileN / 2 : kTileN) * kChunkK * 2; }
+__host__ __device__ constexpr uint32_t exact_stage_bytes(bool stream_a, bool pair) {
+  return (stream_a ? kChunkBytes : 0u) + exact_b_chunk_bytes(pair);
 }
 // everything in dynamic shared memory except the pipeline stages (kernel and host compute the layout from this)
 __host__ __device__ constexpr uint32_t exact_fixed_smem(uint32_t k_chunks, bool stream_a) {
@@ -504,24 +500,15 @@ __device__ __noinline__ void exact_wq_flush(uint32_t* cand_cnt, uint32_t* cand_i
 
 // smem: [A: k_chunks x 16 KB (resident form)][stages: n_stages x ([A chunk] B chunk)]
 //       [warp queues: key | id | lane][barriers][tmem ptr]
-template <bool STREAM_A, bool PAIR, uint32_t TILE_N>
+template <bool STREAM_A, bool PAIR>
 __device__ __forceinline__ void exact_gemm_filter_body(const CUtensorMap* map_q, const CUtensorMap* map_x, const ExactArgs& a) {
   extern __shared__ __align__(1024) uint8_t smem[];
   const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t rank = PAIR ? cluster_ctarank() : 0u;   // CTA within the pair; rank 0 (the leader) issues the MMAs
   const uint32_t n_workers = PAIR ? gridDim.x >> 1 : gridDim.x, worker = PAIR ? blockIdx.x >> 1 : blockIdx.x;
-  // TILE_N = 256 (shipped): two 256-column accumulators, every epilogue warp on every tile.  TILE_N = 128 (measured
-  // alternative, TURDB_EXACT_TILE_N=128): FOUR 128-column accumulators and two alternating sets of eight epilogue warps (set
-  // s takes the tiles with sequence number = s mod 2), so that every accumulator hand-off (commit -> wake -> TMEM load ->
-  // arrive -> wake, ~0.9k cycles against ~1k cycles of MMAs per 256-column tile at K = 128) has three tiles of cover.
-  // Parity-green and slower at every short K tried (128-d L2 4.63 against 3.26 ms): twice the MMA instructions, commits and
-  // barrier round trips per score.
-  constexpr uint32_t kBufs = 512 / TILE_N;                          // accumulator buffers in TMEM
-  constexpr uint32_t kSets = TILE_N == 128 ? 2 : 1;                 // alternating sets of epilogue warps
-  static_assert(TILE_N == 128 || TILE_N == 256, "UMMA N");
-  static_assert((kEpiWarps / kSets) * kEpiCols == 4 * TILE_N, "a set's warps cover the tile: 4 lane quarters x TILE_N columns");
-  constexpr uint32_t kBRows = PAIR ? TILE_N / 2 : TILE_N;          // vector rows this CTA stages per tile
-  constexpr uint32_t stage_bytes = exact_stage_bytes(STREAM_A, PAIR, TILE_N);  // [A chunk |] B chunk
+  constexpr uint32_t kBufs = 512 / kTileN;                          // accumulator buffers in TMEM
+  constexpr uint32_t kBRows = PAIR ? kTileN / 2 : kTileN;          // vector rows this CTA stages per tile
+  constexpr uint32_t stage_bytes = exact_stage_bytes(STREAM_A, PAIR);  // [A chunk |] B chunk
   constexpr uint32_t b_in_stage = STREAM_A ? kChunkBytes : 0;
   constexpr uint32_t kQRows = PAIR ? 2 * kTileM : kTileM;          // queries per work item
   uint8_t* sA = smem;
@@ -545,11 +532,11 @@ __device__ __forceinline__ void exact_gemm_filter_body(const CUtensorMap* map_q,
     }
     for (uint32_t s = 0; s < kBufs; ++s) {
       mbar_init(bar_t_full + 8 * s, 1);
-      mbar_init(bar_t_empty + 8 * s, (PAIR ? 2 : 1) * (kEpiWarps / kSets));  // one arrive per warp of the tile's set (of both CTAs)
+      mbar_init(bar_t_empty + 8 * s, (PAIR ? 2 : 1) * kEpiWarps);  // one arrive per epilogue warp (of both CTAs)
     }
     mbar_fence_init();
   }
-  if (warp == 1) {  // kBufs accumulator buffers x TILE_N FP32 columns = all 512 (in each CTA of a pair)
+  if (warp == 1) {  // kBufs accumulator buffers x kTileN FP32 columns = all 512 (in each CTA of a pair)
     if (PAIR) {
       asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512u)
                    : "memory");
@@ -600,7 +587,7 @@ __device__ __forceinline__ void exact_gemm_filter_body(const CUtensorMap* map_q,
           a_phase ^= 1;
         }
         for (uint32_t t = t0; t < t1; ++t) {
-          const int32_t x_row0 = (int32_t)(t * TILE_N + rank * kBRows);
+          const int32_t x_row0 = (int32_t)(t * kTileN + rank * kBRows);
           for (uint32_t kc = 0; kc < a.k_chunks; ++kc) {
             long long c1 = a.dbg ? clock64() : 0;
             mbar_wait(bar_b_empty + 8 * stage, phase ^ 1);
@@ -641,7 +628,7 @@ __device__ __forceinline__ void exact_gemm_filter_body(const CUtensorMap* map_q,
     if (rank == 0) {
       // instruction descriptor: D=F32, A=B=F16/BF16, both K-major, N, M (cute::UMMA::InstrDescriptor); M = 256 across a pair
       const uint32_t fmt = a.fp16 ? 0u : 1u;  // a_format (bits 7-9) / b_format (bits 10-12): 0 = F16, 1 = BF16
-      const uint32_t idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | ((TILE_N >> 3) << 17) | (((PAIR ? 2 * kTileM : kTileM) >> 4) << 24);
+      const uint32_t idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | ((kTileN >> 3) << 17) | (((PAIR ? 2 * kTileM : kTileM) >> 4) << 24);
       uint32_t stage = 0, phase = 0, a_phase = 0, acc = 0, acc_phase = 0;
       for (uint32_t item = worker; item < a.n_items; item += n_workers) {
         const uint32_t t0 = a.tile_lo + (item / a.n_qblocks) * a.tiles_per_item;
@@ -658,7 +645,7 @@ __device__ __forceinline__ void exact_gemm_filter_body(const CUtensorMap* map_q,
           mbar_wait(bar_t_empty + 8 * acc, acc_phase ^ 1);  // the epilogue (of both CTAs of a pair) has drained this accumulator
           if (a.dbg && lane == 0) atomicAdd(a.dbg + 3, (unsigned long long)(clock64() - c3));
           tc_fence_after();
-          const uint32_t d_tmem = tmem_base + acc * TILE_N;
+          const uint32_t d_tmem = tmem_base + acc * kTileN;
           for (uint32_t kc = 0; kc < a.k_chunks; ++kc) {
             long long c4 = a.dbg ? clock64() : 0;
             mbar_wait(bar_b_full + 8 * stage, phase);
@@ -708,12 +695,11 @@ __device__ __forceinline__ void exact_gemm_filter_body(const CUtensorMap* map_q,
     // per tile — the same work in another order: 128-d 3.32 against 3.19 ms, 768-d 10.36 against 10.20 ms.  At short K the
     // tensor pipe idles on the accumulator hand-offs — commit -> wake -> TMEM load -> arrive -> wake, ~0.9k cycles per
     // 1.05k-cycle tile at 128-d (ncu: pipe 53 % active, the issuer 29 % of its time on bar_t_empty) — which two
-    // 256-column buffers cannot hide.  Four 128-column buffers (TILE_N = 128 below) hide them and still lose: 4.63 against
-    // 3.26 ms at 128-d L2.)
+    // 256-column buffers cannot hide.  Four 128-column buffers, served by two alternating sets of eight warps, hide them and
+    // still lose: 4.63 against 3.26 ms at 128-d L2 — twice the MMA instructions, commits and barrier round trips per score.)
     const uint32_t ew = warp - 2;                    // index among the epilogue warps
     const uint32_t quarter = warp & 3;               // TMEM lane quarter this warp may read (= warp id % 4)
-    const uint32_t set = kSets == 2 ? ew / (kEpiWarps / 2) : 0u;              // which tiles this warp takes (sequence % kSets)
-    const uint32_t cslice = ((ew % (kEpiWarps / kSets)) >> 2) * kEpiCols;     // first tile column of this warp's slice
+    const uint32_t cslice = ((ew % kEpiWarps) >> 2) * kEpiCols;  // first tile column of this warp's slice
     const uint32_t et = threadIdx.x - 64;            // index among the epilogue threads
     const uint32_t lt_mask = (1u << lane) - 1u;
     float* my_key = wq_key + ew * kWq;
@@ -735,15 +721,14 @@ __device__ __forceinline__ void exact_gemm_filter_body(const CUtensorMap* map_q,
       const uint32_t q = q_base + lane;
       const float tau = q < a.nq ? a.thresh[q] : INFINITY;  // rows past the batch never keep anything
       for (uint32_t t = t0; t < t1; ++t, ++seq) {
-        if (kSets == 2 && (seq & 1u) != set) continue;  // the other set's tile
         const uint32_t acc = seq % kBufs, acc_phase = (seq / kBufs) & 1u;
         long long c6 = (a.dbg && et == 0) ? clock64() : 0;
         mbar_wait(bar_t_full + 8 * acc, acc_phase);
         long long c7 = (a.dbg && et == 0) ? clock64() : 0;
         tc_fence_after();
-        const uint32_t n_valid = min(TILE_N, a.n_vec - t * TILE_N);  // columns past the corpus are zero rows
+        const uint32_t n_valid = min(kTileN, a.n_vec - t * kTileN);  // columns past the corpus are zero rows
         uint32_t v[kEpiCols / 32][32];
-        const uint32_t tcol = tmem_base + ((quarter * 32) << 16) + acc * TILE_N + cslice;
+        const uint32_t tcol = tmem_base + ((quarter * 32) << 16) + acc * kTileN + cslice;
         if (a.diag != 1) {
 #pragma unroll
           for (uint32_t cb = 0; cb < kEpiCols / 32; ++cb) tmem_ld_32x32b_x32_nowait(tcol + cb * 32, v[cb]);
@@ -766,7 +751,7 @@ __device__ __forceinline__ void exact_gemm_filter_body(const CUtensorMap* map_q,
           if (a.dense) {  // first slice: no test, no queue — 128-bit stores of the thread's 32 consecutive columns
             if (q < a.nq) {
               const uint32_t c0 = cslice + cb * 32;  // tile column of v[cb][0]
-              const size_t slot = (size_t)q * a.cap + (size_t)(t - a.tile_lo) * TILE_N + c0;
+              const size_t slot = (size_t)q * a.cap + (size_t)(t - a.tile_lo) * kTileN + c0;
               float4* kd = reinterpret_cast<float4*>(a.cand_key + slot);
               uint4* idd = reinterpret_cast<uint4*>(a.cand_id + slot);
 #pragma unroll
@@ -782,7 +767,7 @@ __device__ __forceinline__ void exact_gemm_filter_body(const CUtensorMap* map_q,
                 kv.z = kv.z == kv.z ? kv.z : -INFINITY;
                 kv.w = kv.w == kv.w ? kv.w : -INFINITY;
                 kd[j >> 2] = kv;
-                const uint32_t id0 = t * TILE_N + c0 + j;
+                const uint32_t id0 = t * kTileN + c0 + j;
                 idd[j >> 2] = make_uint4(id0, id0 + 1, id0 + 2, id0 + 3);
               }
             }
@@ -807,7 +792,7 @@ __device__ __forceinline__ void exact_gemm_filter_body(const CUtensorMap* map_q,
                     if (hit) {
                       const uint32_t slot = wq_n + __popc(b & lt_mask);
                       my_key[slot] = key;
-                      my_id[slot] = t * TILE_N + col;
+                      my_id[slot] = t * kTileN + col;
                       my_lane[slot] = lane;
                     }
                     wq_n += __popc(b);
@@ -839,19 +824,19 @@ __device__ __forceinline__ void exact_gemm_filter_body(const CUtensorMap* map_q,
   }
 }
 
-template <bool STREAM_A, uint32_t TILE_N>
+template <bool STREAM_A>
 __global__ void __launch_bounds__(kExactThreads, 1)
 exact_gemm_filter_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_x,
                          const ExactArgs a) {
-  exact_gemm_filter_body<STREAM_A, false, TILE_N>(&map_q, &map_x, a);
+  exact_gemm_filter_body<STREAM_A, false>(&map_q, &map_x, a);
 }
 
 // the two-CTA form: clusters of 2 CTAs (one TPC), grid = 2 x the number of pairs
-template <bool STREAM_A, uint32_t TILE_N>
+template <bool STREAM_A>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kExactThreads, 1)
 exact_gemm_filter_pair_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_x,
                               const ExactArgs a) {
-  exact_gemm_filter_body<STREAM_A, true, TILE_N>(&map_q, &map_x, a);
+  exact_gemm_filter_body<STREAM_A, true>(&map_q, &map_x, a);
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -24,16 +24,13 @@
 
 #include "common.cuh"
 
-// 0: double-buffered list merge (2 x 8 B x ef of shared memory); 1: in-place merge in register batches (half the
-// list memory — what lets 5 queries stay resident per SM at dim 384 — and, batched, also the faster one).
-#ifndef TURDB_MERGE_MODE
-#define TURDB_MERGE_MODE 1
-#endif
+// Measured and dropped: a double-buffered list merge (2 x 8 B x ef of shared memory) — the in-place merge in register
+// batches below needs half the list memory (what lets 5 queries stay resident per SM at dim 384) and is also faster.
 
-// 0: whole vectors arrive by TMA bulk copies (one per vector, mbarrier completion) — the default;
-// 1: by per-thread 16 B cp.async (LDGSTS), 512 B per warp instruction, commit/wait groups.  Measured on B200
-//    (1M x 384 and 1M x 128): the LDGSTS issue stalls for ~2.6k cycles per 8-vector chunk against ~0.9k for
-//    eight bulk copies, 25-33 % slower end to end — kept only as the measured alternative (DESIGN.md §4.1).
+// Measured and dropped: per-thread 16 B cp.async (LDGSTS) gathers instead of one TMA bulk copy per vector — the LDGSTS
+// issue stalls ~2.6k cycles per 8-vector chunk against ~0.9k for eight bulk copies, 25-33 % slower at 1M x 384 and
+// 1M x 128 on B200.
+
 // 1: vectors of a hop that do not fit the first gather round are prefetched into L2 during that round
 #ifndef TURDB_R2_PREFETCH
 #define TURDB_R2_PREFETCH 1
@@ -47,16 +44,9 @@
 #define TURDB_MIN_CTAS 5
 #endif
 
-// 1: FP32 rows are gathered four at a time with TMA tile::gather4 (see team_distances_g4) instead of one bulk copy each.
-//    Measured on B200: correct (parity tests) but slower than the bulk copies (1M x 384: 9.94 vs 8.14 ms; 1M x 128: 5.18 vs
-//    4.74 ms) — the issue phase does not shrink and the reduce over piece-split rows grows.  Off by default.
-#ifndef TURDB_GATHER4
-#define TURDB_GATHER4 0
-#endif
-
-#ifndef TURDB_GATHER_MODE
-#define TURDB_GATHER_MODE 0
-#endif
+// Measured and dropped: gathering FP32 rows four at a time with the TMA tensor copy's four-row gather mode (DESIGN.md §4.1)
+// — parity-green but slower than the bulk copies (1M x 384: 9.94 vs 8.14 ms; 1M x 128: 5.18 vs 4.74 ms on B200): the issue
+// phase does not shrink and the reduce over piece-split rows grows.
 
 // Rows up to this many bytes are traversed by the direct form (one warp per query, hnsw_search_warp_kernel) unless the
 // caller forces a form (turdb_cuda_index_set_traversal_form)
@@ -89,10 +79,6 @@ struct TeamLayout {
   // a vector streams through its slot in n_segs pieces of seg_steps AVX steps (32 B each); the last piece
   // also carries the < 8-element tail.  The quad's accumulators live in registers across pieces.
   uint32_t n_segs, seg_steps;
-  // gather4 staging (g4_pieces != 0): a row travels in g4_pieces column pieces of g4_boxw floats (g4_boxw == 8 mod 32,
-  // so the four rows of a piece sit 32 B apart modulo 128 B: conflict-free quads without padding); a group of 8 slots
-  // = 2 quads x pieces regions of 16 * g4_boxw bytes
-  uint32_t g4_pieces, g4_boxw, g4_tail_pc, g4_tail_off;
   uint32_t hash_bits;  // shared visited table has 1 << hash_bits slots
   // compact table (hash16 != 0): 16-bit entries = (displacement+1) << rem_bits | remainder of a
   // bijective hash of the id, so an entry still identifies exactly one node (exact set, half the bytes)
@@ -127,7 +113,6 @@ struct SearchArgs {
   // rows the traversal gathers: the FP32 arena (row_bytes == ds * 4) or, for the SQ8 kernels, the code arena
   const uint8_t* rows;
   uint32_t row_bytes;        // bytes between rows == bytes copied per row (multiple of 16)
-  const void* row_map;       // device copy of the arena's 2-D tensor map (gather4 staging), or null
   // search_filtered (search.rs:352-398): one bit per node; candidates that do not fit the shared window
   const uint64_t* visible;   // null => unfiltered search
   uint2* f_ovf;              // [CTAs][f_ocap] (distance bits, id) overflow of the candidate window
@@ -171,8 +156,6 @@ struct Team {
   uint32_t stage_u32;
   uint32_t stride, vec_bytes, n_groups, n_segs, seg_steps;
   const uint8_t* rows;       // gather source, vec_bytes apart
-  const void* row_map;       // gather4: tensor map of the arena
-  uint32_t g4_pieces, g4_boxw, g4_tail_pc, g4_tail_off, n_rows;
   uint32_t phases;           // per-warp parity bits of the groups this warp owns
   float qnorm;
   uint32_t c_issue, c_wait, c_comp;  // diagnostics: cycles spent by this warp per phase
@@ -317,160 +300,13 @@ __device__ __forceinline__ void team_distances_whole(const DeviceIndex& ix, Team
   }
 }
 
-// Whole-vector form with per-thread async copies: chunk c is copied AND reduced by its group's owner, so a
-// warp only ever waits on its own commit groups; a warp that owns several staging groups keeps one chunk
-// in flight in each.
-template <int METRIC>
-__device__ __forceinline__ void team_distances_ldgsts(const DeviceIndex& ix, Team& t, uint32_t m) {
-  const uint32_t lane = t.lane, p = lane & 3, G = t.n_groups;
-  const uint32_t nchunks = (m + 7) >> 3;
-  const uint32_t pieces = t.vec_bytes >> 4;
-  auto issue = [&](uint32_t c) {
-    const uint32_t g = t.group_of(c);
-    const uint32_t cnt = min(8u, m - 8 * c);
-    for (uint32_t v = 0; v < cnt; ++v) {
-      const uint32_t id = t.cand_ids[8 * c + v];
-      const uint8_t* src = reinterpret_cast<const uint8_t*>(ix.arena + (size_t)id * ix.ds);
-      const uint32_t dst = t.stage_u32 + (g * 8 + v) * t.stride;
-      for (uint32_t i = lane; i < pieces; i += 32) cp_async16(dst + 16 * i, src + 16 * i);
-    }
-    cp_async_commit();
-  };
-  long long t0 = t.dbg ? clock64() : 0;
-  uint32_t pend = 0;
-  for (uint32_t c = 0; c < min(G, nchunks); ++c)
-    if (t.owns(c)) {
-      issue(c);
-      ++pend;
-    }
-  if (t.dbg) t.c_issue += (uint32_t)(clock64() - t0);
-  for (uint32_t c = 0; c < nchunks; ++c) {
-    const uint32_t g = t.group_of(c);
-    if (!t.owns(c)) continue;
-    const uint32_t slot = 8 * c + (lane >> 2);
-    float nb = 0.f;
-    if (METRIC == kCosine && slot < m) nb = __ldg(ix.norm2 + t.cand_ids[slot]);
-    long long w0 = t.dbg ? clock64() : 0;
-    cp_async_wait_pending(pend - 1);  // the oldest pending group is this chunk
-    --pend;
-    __syncwarp();                     // every lane's pieces of the chunk are visible to the warp
-    long long w1 = t.dbg ? clock64() : 0;
-    t.c_wait += (uint32_t)(w1 - w0);
-    const float* b = reinterpret_cast<const float*>(t.stage + (g * 8 + (lane >> 2)) * t.stride);
-    const float raw = (METRIC == kL2) ? quad_l2sq(t.q, b, ix.dim, p) : quad_dot(t.q, b, ix.dim, p);
-    if (p == 0 && slot < m) {
-      float d = raw;
-      if (METRIC == kIP) d = -raw;  // inner_product_avx2, distance.rs:240-242
-      if (METRIC == kCosine) d = cosine_finish(raw, t.qnorm, nb);
-      if (b[0] == INFINITY) d = INFINITY;  // absent vector
-      t.cand_d[slot] = d;
-    }
-    __syncwarp();                     // the group's slots are free again
-    if (t.dbg) t.c_comp += (uint32_t)(clock64() - w1);
-    if (c + G < nchunks) {
-      issue(c + G);
-      ++pend;
-    }
-  }
-}
-
-#if TURDB_GATHER4
-// gather4 form of the whole-row path (FP32 arena): a hop's bulk copies cost ~100 issue cycles EACH (ELECT / R2UR /
-// UBLKCP per lane); one tile::gather4 instruction moves four rows (x one column piece), so a 24-neighbour hop issues
-// 6 x pieces instructions instead of 24.  Unit (quad qd, piece pc): rows 4qd..4qd+3 of the request, columns
-// [pc * boxw, (pc + 1) * boxw); a quad with fewer than four rows left is padded with row index n — out-of-bounds rows
-// and columns read as zeros, move no data and still count the full box on the barrier (probed: tools/micro).
-template <int METRIC>
-__device__ __forceinline__ void team_distances_g4(const DeviceIndex& ix, Team& t, uint32_t m) {
-  const uint32_t lane = t.lane, p = lane & 3, G = t.n_groups, P = t.g4_pieces, BW = t.g4_boxw;
-  const uint32_t region = 16 * BW, group_bytes = 2 * P * region;
-  const uint32_t nchunks = (m + 7) >> 3;
-  auto unit = [&](uint32_t qd, uint32_t pc, bool prefetch_only) {
-    const uint32_t c = qd >> 1, g = t.group_of(c);
-    int32_t r[4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) r[j] = (4 * qd + j < m) ? (int32_t)t.cand_ids[4 * qd + j] : (int32_t)t.n_rows;
-    if (prefetch_only) {
-      tma_gather4_prefetch(t.row_map, (int32_t)(pc * BW), r[0], r[1], r[2], r[3]);
-    } else {
-      tma_gather4(t.stage_u32 + g * group_bytes + ((qd & 1) * P + pc) * region, t.row_map, (int32_t)(pc * BW), r[0], r[1], r[2],
-                  r[3], t.bar0 + 8 * g);
-    }
-  };
-  auto chunk_bytes = [&](uint32_t c) { return ((min(8u, m - 8 * c) + 3) >> 2) * P * region; };
-  long long t0 = t.dbg ? clock64() : 0;
-  {
-    const uint32_t m1 = min(m, 8 * G);
-    for (uint32_t c = 0; c < min(G, nchunks); ++c)
-      if (t.owns(c) && lane == 0) mbar_expect_tx(t.bar0 + 8 * c, chunk_bytes(c));
-    const uint32_t n_units = ((m1 + 3) >> 2) * P;
-    const uint32_t i = t.warp + t.n_warps * lane;  // units dealt to all warps, the leader included
-    if (i < n_units) unit(i / P, i % P, false);
-#if TURDB_R2_PREFETCH
-    const uint32_t n2 = ((m - m1 + 3) >> 2) * P;
-    if (t.warp == 0 && t.n_warps >= 3 && lane < n2) unit((m1 >> 2) + lane / P, lane % P, true);
-#endif
-  }
-  if (t.dbg) t.c_issue += (uint32_t)(clock64() - t0);
-  const uint32_t steps = ix.dim >> 3, spp = BW >> 3;
-  for (uint32_t c = 0; c < nchunks; ++c) {
-    const uint32_t g = t.group_of(c);
-    if (!t.owns(c)) continue;
-    const uint32_t v = lane >> 2, slot = 8 * c + v;
-    float nb = 0.f;
-    if (METRIC == kCosine && slot < m) nb = __ldg(ix.norm2 + t.cand_ids[slot]);
-    long long w0 = t.dbg ? clock64() : 0;
-    mbar_wait(t.bar0 + 8 * g, (t.phases >> g) & 1u);
-    long long w1 = t.dbg ? clock64() : 0;
-    t.c_wait += (uint32_t)(w1 - w0);
-    t.phases ^= (1u << g);
-    const uint8_t* base = t.stage + g * group_bytes + (v >> 2) * P * region + (v & 3) * BW * 4;
-    uint64_t acc = 0ull;
-    for (uint32_t pc = 0, s0 = 0; s0 < steps; ++pc, s0 += spp) {
-      const uint32_t ns = min(spp, steps - s0);
-      const uint64_t* av = reinterpret_cast<const uint64_t*>(t.q + 8 * s0) + p;
-      const uint64_t* bv = reinterpret_cast<const uint64_t*>(base + pc * region) + p;
-      acc = (METRIC == kL2) ? quad_accum<true>(acc, av, bv, ns) : quad_accum<false>(acc, av, bv, ns);
-    }
-    const float* bt = reinterpret_cast<const float*>(base + t.g4_tail_pc * region) + t.g4_tail_off;
-    const float raw = (METRIC == kL2) ? quad_finish<true>(acc, t.q + 8 * steps, bt, ix.dim & 7)
-                                      : quad_finish<false>(acc, t.q + 8 * steps, bt, ix.dim & 7);
-    if (p == 0 && slot < m) {
-      float d = raw;
-      if (METRIC == kIP) d = -raw;
-      if (METRIC == kCosine) d = cosine_finish(raw, t.qnorm, nb);
-      if (*reinterpret_cast<const float*>(base) == INFINITY) d = INFINITY;  // absent vector
-      t.cand_d[slot] = d;
-    }
-    __syncwarp();
-    if (t.dbg) t.c_comp += (uint32_t)(clock64() - w1);
-    if (c + G < nchunks) {  // second round: this chunk's owner issues the next chunk of its group
-      const uint32_t c2 = c + G, nq2 = (min(8u, m - 8 * c2) + 3) >> 2;
-      if (lane == 0) mbar_expect_tx(t.bar0 + 8 * g, chunk_bytes(c2));
-      __syncwarp();
-      if (lane < nq2 * P) unit(2 * c2 + lane / P, lane % P, false);
-    }
-  }
-}
-#endif
-
 template <int METRIC, bool SQ8>
 __device__ __forceinline__ void team_distances(const DeviceIndex& ix, Team& t, uint32_t m) {
   if (SQ8) {  // code rows are short: always the whole-row form (the host never splits them)
     team_distances_whole<METRIC, true>(ix, t, m);
     return;
   }
-#if TURDB_GATHER4
-  if (t.g4_pieces) {
-    team_distances_g4<METRIC>(ix, t, m);
-    return;
-  }
-#endif
-#if TURDB_GATHER_MODE == 1
-  if (t.n_segs == 1) team_distances_ldgsts<METRIC>(ix, t, m);
-#else
   if (t.n_segs == 1) team_distances_whole<METRIC, false>(ix, t, m);
-#endif
   else team_distances_pieces<METRIC>(ix, t, m);
 }
 
@@ -497,7 +333,8 @@ __device__ __forceinline__ float leader_request(const DeviceIndex& ix, Team& t, 
 // A quad of lanes owns one neighbour row per pass (8 rows per pass); lane p of the quad loads the 8 bytes
 // (elements 8t+2p, 8t+2p+1) of AVX step t with one LDG.64, so the quad reads one 32 B sector per step and every
 // lane's accumulator is exactly the reference's AVX2 lane pair (distance.rs:105-129).  A row streams through in
-// column chunks of 16 steps (128 floats, 16 registers pairs); two chunks are in flight per warp.
+// units of 8 steps (64 floats, 8 register pairs per lane); one unit is in flight per warp, and the rest of the request
+// is prefetched into L2 (TURDB_DIRECT_PREFETCH).
 // step S of a unit: base + 32 S bytes, the offset folded into the instruction (a register operand per load would
 // cost an address register pair each)
 template <int S, int US>
@@ -512,21 +349,13 @@ struct LoadSteps<US, US> {
   static __device__ __forceinline__ void run(uint64_t (&)[US], const uint64_t*, uint32_t) {}
 };
 
-// steps (of 8 floats) per unit and units in flight per warp: registers for the landing zone = 2 * US * NBUF
-// 1: rows of the speculated next hop are prefetched into L2 during the current hop (rows up to ..._MAX_ROW bytes).
-// Measured on B200 (r02, 2M x 128 clustered / 1M x 128 SIFT-like): no gain in the direct form (2.648 vs 2.647 ms), 5 %
-// slower in the staged form (3.16 vs 3.00 ms) — the 128-d kernel waits on dependent instructions, not on the rows.  Off.
-#ifndef TURDB_SPEC_PREFETCH
-#define TURDB_SPEC_PREFETCH 0
-#endif
-#ifndef TURDB_SPEC_PREFETCH_MAX_ROW
-#define TURDB_SPEC_PREFETCH_MAX_ROW 1024
-#endif
+// Measured and dropped: prefetching the rows of the speculated next hop into L2 during the current hop — no gain in the
+// direct form (2.648 vs 2.647 ms), 5 % slower in the staged form (3.16 vs 3.00 ms) at 2M x 128 clustered / 1M x 128
+// SIFT-like on B200: the 128-d kernel waits on dependent instructions, not on the rows.
+// Measured and dropped: direct-form landing zones of 16 steps x 1, 8 x 2, 8 x 3 and 4 x 2 units in flight — all slower
+// or spilling against 8 x 1.
 #ifndef TURDB_DIRECT_DBG
 #define TURDB_DIRECT_DBG 0
-#endif
-#ifndef TURDB_DIRECT_US
-#define TURDB_DIRECT_US 8
 #endif
 // 1: rows of a request beyond the first pass (candidates 8..m-1) are prefetched into L2 when the request starts,
 // one 128 B line per lane and instruction: their loads then pay an L2 hit instead of a second and third DRAM
@@ -534,28 +363,25 @@ struct LoadSteps<US, US> {
 #ifndef TURDB_DIRECT_PREFETCH
 #define TURDB_DIRECT_PREFETCH 1
 #endif
-#ifndef TURDB_DIRECT_NBUF
-#define TURDB_DIRECT_NBUF 1
-#endif
 
 template <int METRIC, typename F>
 __device__ __forceinline__ float warp_request(const DeviceIndex& ix, Team& t, uint32_t m, F&& overlap) {
-  constexpr int US = TURDB_DIRECT_US, NBUF = TURDB_DIRECT_NBUF;
+  constexpr int US = 8;  // steps (of 8 floats) per unit: the landing zone is 2 * US registers
   const uint32_t lane = t.lane, p = lane & 3, qd = lane >> 2;
   const uint32_t steps = ix.dim >> 3, ntail = ix.dim & 7;
   const uint32_t nch = max(1u, (steps + US - 1) / US);
   const bool full = steps != 0 && steps % US == 0;  // every unit carries US steps: the loops below run unpredicated
   const uint32_t npass = (m + 7) >> 3, nunits = npass * nch;
-  uint64_t b[NBUF][US];
+  uint64_t b[US];
   __syncwarp();  // cand_ids[0..m) were written by lanes 0..m-1; every quad reads them (the staged form has a CTA barrier here)
   // Quads beyond the request's last candidate gather (and reduce) that last candidate again: every lane then runs
   // the same unpredicated instruction stream; their result is discarded.
   uint32_t l_pass = 0, l_ch = 0;  // next unit to load
-  auto load = [&](uint64_t (&bb)[US]) {
+  auto load = [&] {
     const uint32_t id = t.cand_ids[min(8 * l_pass + qd, m - 1)];
     const uint64_t* src = reinterpret_cast<const uint64_t*>(t.rows + (size_t)id * t.vec_bytes) + 4 * US * l_ch + p;
-    if (full) LoadSteps<0, US>::run(bb, src, US);
-    else LoadSteps<0, US>::run(bb, src, min((uint32_t)US, steps - US * l_ch));
+    if (full) LoadSteps<0, US>::run(b, src, US);
+    else LoadSteps<0, US>::run(b, src, min((uint32_t)US, steps - US * l_ch));
     if (++l_ch == nch) {
       l_ch = 0;
       ++l_pass;
@@ -564,30 +390,30 @@ __device__ __forceinline__ float warp_request(const DeviceIndex& ix, Team& t, ui
   uint32_t c_pass = 0, c_ch = 0;  // next unit to reduce
   uint64_t acc = 0ull;
   float out = INFINITY, first = 0.f;
-  auto consume = [&](const uint64_t (&bb)[US]) {
+  auto consume = [&] {
     const uint64_t* av = reinterpret_cast<const uint64_t*>(t.q + 8 * US * c_ch) + p;
     if (full) {
-      if (c_ch == 0) first = __uint_as_float((uint32_t)bb[0]);  // element 0 of the row, in the quad's lane 0
+      if (c_ch == 0) first = __uint_as_float((uint32_t)b[0]);  // element 0 of the row, in the quad's lane 0
 #pragma unroll
       for (int s = 0; s < US; ++s) {
         if (METRIC == kL2) {
-          const uint64_t d = sub2(av[4 * s], bb[s]);
+          const uint64_t d = sub2(av[4 * s], b[s]);
           acc = fma2(d, d, acc);
         } else {
-          acc = fma2(av[4 * s], bb[s], acc);
+          acc = fma2(av[4 * s], b[s], acc);
         }
       }
     } else {
       const uint32_t ns = min((uint32_t)US, steps - US * c_ch);
-      if (c_ch == 0) first = ns ? __uint_as_float((uint32_t)bb[0]) : 0.f;
+      if (c_ch == 0) first = ns ? __uint_as_float((uint32_t)b[0]) : 0.f;
 #pragma unroll
       for (int s = 0; s < US; ++s)
         if ((uint32_t)s < ns) {
           if (METRIC == kL2) {
-            const uint64_t d = sub2(av[4 * s], bb[s]);
+            const uint64_t d = sub2(av[4 * s], b[s]);
             acc = fma2(d, d, acc);
           } else {
-            acc = fma2(av[4 * s], bb[s], acc);
+            acc = fma2(av[4 * s], b[s], acc);
           }
         }
     }
@@ -621,14 +447,12 @@ __device__ __forceinline__ float warp_request(const DeviceIndex& ix, Team& t, ui
       ++c_pass;
     }
   };
-#pragma unroll
-  for (int i = 0; i < NBUF; ++i)
-    if ((uint32_t)i < nunits) load(b[i]);
+  if (nunits != 0) load();
 #if TURDB_DIRECT_PREFETCH
-  if (nunits > (uint32_t)NBUF) {
-    // everything the first NBUF units do not cover is pulled into L2 now, one 128 B line per lane and instruction
-    // (whole rows of the later candidates; with rows longer than the buffers, the rest of every row)
-    const uint32_t r0 = nch > (uint32_t)NBUF ? 0u : 8u * ((uint32_t)NBUF / nch);
+  if (nunits > 1) {
+    // everything the first unit does not cover is pulled into L2 now, one 128 B line per lane and instruction
+    // (whole rows of the later candidates; with rows longer than one unit, the rest of every row)
+    const uint32_t r0 = nch == 1 ? 8u : 0u;
     const uint32_t lpr = ((t.vec_bytes + 127) >> 7) + ((t.vec_bytes & 127) ? 1u : 0u);  // lines a row can touch
     const uint32_t sh = 32 - __clz(lpr - 1), total = (m - min(m, r0)) << sh;             // rounded up to a power of two
     for (uint32_t j = lane; j < total; j += 32) {
@@ -640,13 +464,9 @@ __device__ __forceinline__ float warp_request(const DeviceIndex& ix, Team& t, ui
   }
 #endif
   overlap();
-  for (uint32_t u = 0; u < nunits; u += NBUF) {
-#pragma unroll
-    for (int i = 0; i < NBUF; ++i)
-      if (u + i < nunits) {
-        consume(b[i]);
-        if (u + i + NBUF < nunits) load(b[i]);
-      }
+  for (uint32_t u = 0; u < nunits; ++u) {
+    consume();
+    if (u + 1 < nunits) load();
   }
   __syncwarp();  // all reads of cand_ids are done before the caller reuses it
   return lane < m ? out : INFINITY;
@@ -882,12 +702,6 @@ __device__ __forceinline__ void hnsw_search_body(const SearchArgs& a) {
   t.stride = a.lay.stride;
   t.vec_bytes = a.lay.vec_bytes;
   t.rows = a.rows;
-  t.row_map = a.row_map;
-  t.g4_pieces = a.lay.g4_pieces;
-  t.g4_boxw = a.lay.g4_boxw;
-  t.g4_tail_pc = a.lay.g4_tail_pc;
-  t.g4_tail_off = a.lay.g4_tail_off;
-  t.n_rows = (uint32_t)a.ix.n;
   t.n_groups = a.lay.n_groups;
   t.n_segs = a.lay.n_segs;
   t.seg_steps = a.lay.seg_steps;
@@ -1247,17 +1061,6 @@ __device__ __forceinline__ void hnsw_search_body(const SearchArgs& a) {
           const uint32_t nm = __ballot_sync(kFullMask, sp_inserted);
           sp_m = __popc(nm);
           if (sp_inserted) cand_next[__popc(nm & ((1u << lane) - 1))] = row_nid;
-#if TURDB_SPEC_PREFETCH
-          // short rows: the kernel is latency-bound, so the rows hop h+1 will most likely gather (the speculation holds
-          // ~85 % of the time) are pulled into L2 now, one 128 B line per instruction and lane — hop h+1's loads then pay
-          // an L2 hit.  A wrong guess costs the DRAM bytes of those rows (counted in roofline.traffic, not in the
-          // algorithmic bytes).
-          if (sp_inserted && t.vec_bytes <= TURDB_SPEC_PREFETCH_MAX_ROW) {
-            const uintptr_t r0 = reinterpret_cast<uintptr_t>(t.rows + (size_t)row_nid * t.vec_bytes);
-            for (uintptr_t pa = r0 & ~(uintptr_t)127; pa < r0 + t.vec_bytes; pa += 128)
-              asm volatile("prefetch.global.L2 [%0];" ::"l"(pa));
-          }
-#endif
           sp_node = row_node;
           sp_valid = true;
         });
@@ -1298,31 +1101,6 @@ __device__ __forceinline__ void hnsw_search_body(const SearchArgs& a) {
           rank += (db < d || (db == d && bsrc < lane)) ? 1u : 0u;
         }
         __syncwarp();
-#if TURDB_MERGE_MODE == 0
-        // double-buffered: every old entry moves right by the number of new entries inserted at or before it
-        for (uint32_t i = lane; i < len; i += 32) {
-          uint32_t sft = 0;
-          for (uint32_t j = 0; j < mp; ++j) sft += (tmp_ub[j] <= i) ? 1u : 0u;
-          const uint32_t np = i + sft;
-          if (np < ef) {
-            B_d[np] = A_d[i];
-            B_id[np] = A_id[i];
-          }
-        }
-        uint32_t my_np = 0xFFFFFFFFu;
-        if (elig) {
-          const uint32_t np = ub + rank;
-          if (np < ef) {
-            B_d[np] = d;
-            B_id[np] = cid;
-            my_np = np;
-          }
-        }
-        {
-          float* td = A_d; A_d = B_d; B_d = td;
-          uint32_t* ti = A_id; A_id = B_id; B_id = ti;
-        }
-#else
         // in place, from the top down in batches of kMergeBatch 32-entry blocks: a batch is read into registers, the
         // warp synchronises, the batch is written at its shifted positions (always >= the old ones, and the
         // batches above have already moved), the warp synchronises
@@ -1365,7 +1143,6 @@ __device__ __forceinline__ void hnsw_search_body(const SearchArgs& a) {
             my_np = np;
           }
         }
-#endif
         scan_from = min(scan_from, __reduce_min_sync(kFullMask, my_np));
         len = min(len + mp, ef);
         __syncwarp();

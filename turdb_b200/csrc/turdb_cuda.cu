@@ -71,8 +71,6 @@ struct turdb_cuda_index {
   uint8_t* d_up_cnt = nullptr;
   uint32_t* d_up_owner = nullptr;
   uint64_t cap_n = 0, cap_slots = 0;       // allocated nodes / upper slots of every per-node / per-slot array (>= n, n_up_slots)
-  void* d_row_map = nullptr;               // device copy of the arena's gather4 tensor map (TURDB_GATHER4 builds)
-  uint32_t g4_boxw = 0;
   uint8_t* d_arena_sq8 = nullptr;          // SQ8 rows: dim codes | pad | min | scale, sq8_row_bytes apart (enable_sq8)
   float* d_norm2_sq8 = nullptr;            // dot(decode(x), decode(x)) per row, AVX2 lane order
   uint32_t sq8_row_bytes = 0;
@@ -256,7 +254,6 @@ int32_t turdb_cuda_index_destroy(turdb_cuda_index* idx) {
     cudaFree(idx->d_l0_cnt);
     cudaFree(idx->d_up_cnt);
     cudaFree(idx->d_up_owner);
-    cudaFree(idx->d_row_map);
     cudaFree(idx->d_arena_sq8);
     cudaFree(idx->d_norm2_sq8);
     cudaFree(idx->d_arena_bf16);
@@ -595,7 +592,7 @@ int32_t turdb_cuda_index_profile_read(turdb_cuda_index* idx, float* main_ms, flo
 // n_slots == 0: the direct form (one warp per query, no staging)
 static TeamLayout make_layout(uint32_t dim, uint32_t ds, uint32_t ef, uint32_t hash_bits, uint32_t n_slots, uint32_t n_segs,
                               bool global_visited, uint64_t n_nodes, bool filtered = false, uint32_t sq8_row_bytes = 0,
-                              uint32_t g4_boxw = 0, bool entries32 = false) {
+                              bool entries32 = false) {
   TeamLayout L{};
   L.vec_bytes = sq8_row_bytes ? sq8_row_bytes : ds * 4;
   const uint32_t steps = dim >> 3;
@@ -614,27 +611,14 @@ static TeamLayout make_layout(uint32_t dim, uint32_t ds, uint32_t ef, uint32_t h
   // [0] mbarriers, [32] control words, [64] cand_ids[32] cand_d[32] tmp_ub[32] cand_next[32], [576] result list: fixed
   // offsets (kOffBar .. kOffList); then the filtered window, the query, the visited table, the staging slots
   uint32_t off = kOffList;
-  off += (filtered || TURDB_MERGE_MODE == 0) ? ef * 16 : ef * 8;  // result list (x2 when double-buffered)
+  off += filtered ? ef * 16 : ef * 8;  // result list (x2: the filtered search double-buffers it)
   L.off_clist = off; off += filtered ? ef * 16 : 0;       // search_filtered: candidate window (double-buffered)
   off = (off + 15) & ~15u;
   L.off_q = off;     off += (ds * 4 + 15) & ~15u;
   L.off_hash = off;  off += global_visited ? 0 : ((L.hash16 ? 2u : 4u) << hash_bits);
   off = (off + 127) & ~127u;
   L.off_stage = off;
-  if (g4_boxw && !sq8_row_bytes && L.n_segs == 1 && n_slots) {
-    L.g4_boxw = g4_boxw;
-    L.g4_pieces = (ds + g4_boxw - 1) / g4_boxw;
-    const uint32_t e0 = steps * 8;  // first element of the < 8-element tail
-    L.g4_tail_pc = e0 / g4_boxw;
-    L.g4_tail_off = e0 - L.g4_tail_pc * g4_boxw;
-    if (L.g4_tail_pc >= L.g4_pieces) {  // dim % 8 == 0 and the row ends exactly at a piece boundary: never dereferenced
-      L.g4_tail_pc = L.g4_pieces - 1;
-      L.g4_tail_off = 0;
-    }
-    off += L.n_groups * 2 * L.g4_pieces * 16 * g4_boxw;
-  } else {
-    off += n_slots * L.stride;
-  }
+  off += n_slots * L.stride;
   L.team_bytes = (off + 127) & ~127u;
   return L;
 }
@@ -679,8 +663,6 @@ __global__ void fill_empty_results_kernel(uint64_t* rows, uint32_t* nodes, float
   if (i < nq) counts[i] = 0;
   if (stats && i < (uint64_t)nq * 4) stats[i] = 0;
 }
-
-[[maybe_unused]] static int32_t ensure_row_map(turdb_cuda_index* idx);  // defined after the tensor-map helpers (exact_abi.inl)
 
 // the insert path's searches (graph_insert.inl): nodes [first, first + nq) against the graph built so far
 struct InsertSpec {
@@ -768,19 +750,12 @@ static int32_t search_batch_device_impl(turdb_cuda_index* idx, const float* d_qu
   const bool direct = !sq8 && (tm == 2 || (tm == 0 && ds * 4 <= TURDB_DIRECT_MAX_ROW_BYTES && rows_per_hop > 0.0 &&
                                            rows_per_hop <= TURDB_DIRECT_MAX_ROWS_PER_HOP));
   uint32_t warps = direct ? 1u : (tw ? std::min(tw, 4u) : 0u);  // staged team size (0: chosen below)
-  uint32_t g4w = 0;
-#if TURDB_GATHER4
-  if (!sq8 && !direct && ds <= 4 * 232) {
-    if (int32_t rc = ensure_row_map(idx); rc != TURDB_OK) return rc;
-    g4w = idx->g4_boxw;
-  }
-#endif
   const uint32_t rb8 = sq8 ? idx->sq8_row_bytes : 0;
   TeamLayout lay{};
   bool auto_warps = false;
   if (direct) {
-    lay = make_layout(dim, ds, ef, hash_bits, 0, 1, false, nn, filt, 0, 0, entries32);
-    while (lay.team_bytes > budget && hash_bits > 8) lay = make_layout(dim, ds, ef, --hash_bits, 0, 1, false, nn, filt, 0, 0, entries32);
+    lay = make_layout(dim, ds, ef, hash_bits, 0, 1, false, nn, filt, 0, entries32);
+    while (lay.team_bytes > budget && hash_bits > 8) lay = make_layout(dim, ds, ef, --hash_bits, 0, 1, false, nn, filt, 0, entries32);
   } else {
     uint32_t slots = ts, segs = tg;
     if (sq8) {
@@ -802,7 +777,7 @@ static int32_t search_batch_device_impl(turdb_cuda_index* idx, const float* d_qu
       for (uint32_t cg = tg ? tg : 1; cg <= (tg ? tg : 8); ++cg) {
         uint32_t best_occ = 0;
         for (uint32_t cs = ts ? ts : 8; cs <= (ts ? ts : 32); cs += 8) {
-          TeamLayout L = make_layout(dim, ds, ef, hash_bits, cs, cg, false, nn, filt, rb8, g4w, entries32);
+          TeamLayout L = make_layout(dim, ds, ef, hash_bits, cs, cg, false, nn, filt, rb8, entries32);
           if (L.n_segs != cg || L.team_bytes > budget) continue;
           if (cg > 1 && L.seg_steps * 32 < 512) continue;
           const uint32_t occ = std::min(8u, sm_bytes / (L.team_bytes + 1024));
@@ -819,7 +794,7 @@ static int32_t search_batch_device_impl(turdb_cuda_index* idx, const float* d_qu
       slots = bs;
       segs = bg;
     }
-    lay = make_layout(dim, ds, ef, hash_bits, slots, segs, false, nn, filt, rb8, g4w, entries32);
+    lay = make_layout(dim, ds, ef, hash_bits, slots, segs, false, nn, filt, rb8, entries32);
     // Team size: warp 0 leads (control flow + speculative preparation of the next hop), the others gather and
     // reduce; every warp takes a share of a hop's bulk-copy issue.  Resident queries per SM come first (the
     // kernel is latency-bound); among equal residency the larger team wins (shorter issue phase).
@@ -828,11 +803,11 @@ static int32_t search_batch_device_impl(turdb_cuda_index* idx, const float* d_qu
       warps = 4;
     }
     while (lay.team_bytes > budget && lay.n_segs < 16 && lay.seg_steps > 8)
-      lay = make_layout(dim, ds, ef, hash_bits, lay.n_groups * 8, lay.n_segs + 1, false, nn, filt, rb8, g4w, entries32);
+      lay = make_layout(dim, ds, ef, hash_bits, lay.n_groups * 8, lay.n_segs + 1, false, nn, filt, rb8, entries32);
     while (lay.team_bytes > budget && lay.n_groups > 1)
-      lay = make_layout(dim, ds, ef, hash_bits, lay.n_groups * 8 - 8, lay.n_segs, false, nn, filt, rb8, g4w, entries32);
+      lay = make_layout(dim, ds, ef, hash_bits, lay.n_groups * 8 - 8, lay.n_segs, false, nn, filt, rb8, entries32);
     while (lay.team_bytes > budget && hash_bits > 8)
-      lay = make_layout(dim, ds, ef, --hash_bits, lay.n_groups * 8, lay.n_segs, false, nn, filt, rb8, g4w, entries32);
+      lay = make_layout(dim, ds, ef, --hash_bits, lay.n_groups * 8, lay.n_segs, false, nn, filt, rb8, entries32);
   }
   if (lay.team_bytes > budget)
     return fail(TURDB_ERR_UNSUPPORTED, "dim %u / ef %u need %u B of shared memory per query (> %u)", idx->ix.dim, ef, lay.team_bytes, budget);
@@ -861,8 +836,8 @@ static int32_t search_batch_device_impl(turdb_cuda_index* idx, const float* d_qu
 
   // fallback pass geometry (queries whose visited table or filtered-candidate buffer filled): same form, one bit
   // per node in global memory; its filtered-candidate buffer holds every node, so it cannot fail
-  TeamLayout glay = direct ? make_layout(dim, ds, ef, 8, 0, 1, true, nn, filt, 0, 0)
-                           : make_layout(dim, ds, ef, 8, lay.n_groups * 8, lay.n_segs, true, nn, filt, rb8, g4w);
+  TeamLayout glay = direct ? make_layout(dim, ds, ef, 8, 0, 1, true, nn, filt, 0)
+                           : make_layout(dim, ds, ef, 8, lay.n_groups * 8, lay.n_segs, true, nn, filt, rb8);
   const uint32_t vis_words = (uint32_t)(((nn + 31) / 32 + 3) & ~3ull);
   uint32_t fb_ctas = (uint32_t)std::min<uint32_t>((uint32_t)idx->num_sms, nq);
   const uint32_t f_ocap_main = filt ? (uint32_t)std::min<uint64_t>(nn, 32768) : 0u;
@@ -921,7 +896,6 @@ static int32_t search_batch_device_impl(turdb_cuda_index* idx, const float* d_qu
   a.vis_words = 0;
   a.dbg = idx->d_dbg;
   a.visible = d_vis_live ? d_vis_live : (d_visible ? d_visible : d_live);
-  a.row_map = lay.g4_pieces ? idx->d_row_map : nullptr;
   a.rows = sq8 ? idx->d_arena_sq8 : reinterpret_cast<const uint8_t*>(idx->d_arena);
   a.row_bytes = lay.vec_bytes;
   if (sq8) a.ix.norm2 = idx->d_norm2_sq8;  // cosine's norm_b chain runs over the decoded row
@@ -1128,28 +1102,6 @@ extern "C" int32_t turdb_cuda_index_gather_probe(turdb_cuda_index* idx, uint32_t
 // exact path + merge entry points live in exact_search.cuh / below
 #include "exact_abi.inl"
 
-// The arena as a 2-D FP32 tensor [n][ds] with box {boxw, 1} for TMA tile::gather4 (team_distances_g4).  boxw == 8 (mod
-// 32) floats keeps the four rows of a piece 32 B apart modulo 128 B in shared memory; <= 4 pieces per row.
-[[maybe_unused]] static int32_t ensure_row_map(turdb_cuda_index* idx) {
-  std::lock_guard<std::mutex> lk(idx->mu);
-  if (idx->d_row_map || idx->ix.n == 0) return TURDB_OK;
-  EncodeTiledFn enc = get_encode_tiled();
-  if (!enc) return fail(TURDB_ERR_CUDA, "cuTensorMapEncodeTiled unavailable");
-  const uint32_t ds = idx->ix.ds, pieces = (ds + 231) / 232, need = (ds + pieces - 1) / pieces;
-  const uint32_t boxw = need <= 8 ? 8 : ((need - 8 + 31) / 32) * 32 + 8;
-  CUtensorMap map;
-  cuuint64_t dims[2] = {ds, idx->ix.n};
-  cuuint64_t strides[1] = {(cuuint64_t)ds * 4};
-  cuuint32_t box[2] = {boxw, 1};
-  cuuint32_t estr[2] = {1, 1};
-  if (enc(&map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, idx->d_arena, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-          CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-    return fail(TURDB_ERR_CUDA, "cuTensorMapEncodeTiled failed for the arena (ds %u, box %u)", ds, boxw);
-  CUDA_TRY(cudaMalloc(&idx->d_row_map, sizeof(CUtensorMap)));
-  CUDA_TRY(cudaMemcpy(idx->d_row_map, &map, sizeof(CUtensorMap), cudaMemcpyHostToDevice));
-  idx->g4_boxw = boxw;
-  return TURDB_OK;
-}
 #include "sql_topk.inl"
 #include "sql_range.inl"
 #include "hnsw_file.inl"
