@@ -164,6 +164,35 @@ int32_t turdb_cuda_index_insert(turdb_cuda_index* idx, const turdb_cuda_build_pa
  */
 int32_t turdb_cuda_index_delete(turdb_cuda_index* idx, uint64_t n, const uint32_t* node_ids, uint64_t* out_n_deleted);
 
+/*
+ * Removes the deleted nodes (turdb_cuda_index_delete) from idx: live nodes keep their relative order and are renumbered
+ * 0 .. n_live - 1; the lists that pointed at a deleted node are repaired; the live bitmap is released, so every read
+ * path runs the launches of an index that never had a delete.  A documented extension (the reference's vacuum is not
+ * restated); the tests restate the same rule on the CPU (tests/compact_reference.py):
+ *   - Rows (vector, row id, level, norm, SQ8 row and norm after enable_sq8) move to their new ids; up_base is the
+ *     exclusive prefix sum of the live nodes' levels (INVALID for level 0), and the insert path's per-list state is
+ *     rebuilt, so turdb_cuda_index_insert works afterwards.  The exact path's 16-bit copies are dropped and rebuilt by
+ *     the next exact or SQL call, as after insert.
+ *   - A list without a deleted id is kept verbatim, in new ids.  A list of live node p at level l holding a deleted id
+ *     becomes select_neighbors_heuristic(p, C, cap) (operations.rs:181-233, as the insert path's reference-intent
+ *     back-link uses it; cap 32 at level 0, 16 above) over C = p's live neighbours at l in stored order, then, for each
+ *     deleted neighbour d in p's stored order, d's live neighbours at l in stored order (nothing if d lacks level l);
+ *     first occurrence kept, p excluded.  C is sorted stably ascending by squared L2 to p (AVX2 lane order, whatever the
+ *     metric; NaN as +inf, ties in C's order); the walk and the back-fill follow that order.  Every repaired list is
+ *     computed from the graph as it stood before the call, so the result does not depend on launch order.
+ *   - Entry: a live entry keeps its place (new id, same max_level); a deleted entry is replaced by the live node of the
+ *     highest level (lowest new id among ties), and max_level becomes its level.  Every node deleted: an empty index
+ *     (n = 0, entry TURDB_INVALID_NODE, max_level 0) that a later insert fills like any empty index.
+ *   - .hnsw tombstones (hnsw_file_upload) are live nodes; compaction leaves them alone.
+ *   - out_old_to_new (nullable): n entries, n = the node count before the call; each node's new id, or
+ *     TURDB_INVALID_NODE for a deleted node.  out_n (nullable): the node count after the call.
+ *   - No deletion (never deleted, or every deleted node already removed): writes the identity map and changes nothing.
+ *   - Concurrency: a WRITER call, like insert.  Every allocation happens before anything the index answers from
+ *     changes; on failure (TURDB_ERR_OUT_OF_MEMORY, TURDB_ERR_CUDA) the index is as before.  The device is synchronised
+ *     before the old buffers are freed.
+ */
+int32_t turdb_cuda_index_compact(turdb_cuda_index* idx, uint32_t* out_old_to_new, uint64_t* out_n);
+
 /* The index's graph as flat host arrays (the turdb_cuda_graph layout; counts = valid ids per row); every pointer is
  * nullable.  up_adj / up_cnt hold *n_up_slots rows (call once with only n_up_slots to size them). */
 int32_t turdb_cuda_index_export_graph(turdb_cuda_index* idx, float* vectors, uint64_t* row_ids, uint8_t* levels,

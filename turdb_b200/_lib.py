@@ -56,7 +56,7 @@ EXPORTS = [
     "turdb_cuda_index_enable_sq8", "turdb_cuda_search_batch_sq8_device", "turdb_cuda_shards_search_batch",
     "turdb_cuda_index_build", "turdb_cuda_index_export_graph", "turdb_cuda_index_insert",
     "turdb_cuda_sql_range_batch", "turdb_cuda_sql_range_batch_device", "turdb_cuda_sql_range_topk_batch",
-    "turdb_cuda_sql_range_topk_batch_device", "turdb_cuda_index_delete",
+    "turdb_cuda_sql_range_topk_batch_device", "turdb_cuda_index_delete", "turdb_cuda_index_compact",
 ]
 
 _lib = None
@@ -108,6 +108,7 @@ def load():
     L.turdb_cuda_index_build.argtypes = [C.POINTER(BuildParams), u64, pf, pu64, C.POINTER(C.c_double), i32, C.POINTER(vp)]
     L.turdb_cuda_index_insert.argtypes = [vp, C.POINTER(BuildParams), u64, pf, pu64, C.POINTER(C.c_double)]
     L.turdb_cuda_index_delete.argtypes = [vp, u64, pu32, pu64]
+    L.turdb_cuda_index_compact.argtypes = [vp, pu32, pu64]
     L.turdb_cuda_index_export_graph.argtypes = [vp, pf, pu64, pu8, pu32, pu8, pu32, pu32, pu8, pu32, pu32, pu64]
     L.turdb_cuda_hnsw_file_open.argtypes = [C.c_char_p, C.POINTER(vp)]
     L.turdb_cuda_hnsw_file_open_memory.argtypes = [pu8, u64, C.POINTER(vp)]

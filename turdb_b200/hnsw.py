@@ -190,6 +190,19 @@ class CudaHnswIndex:
                                                    C.byref(out)))
         return int(out.value)
 
+    def compact(self) -> np.ndarray:
+        """Remove the deleted nodes (turdb_cuda_index_compact): live nodes keep their order and are renumbered 0 ..
+        n_live - 1, the lists through deleted nodes are repaired, and every read path then runs as on an index that never
+        had a delete.  Returns the old -> new node id map (uint32 [node count before the call]; INVALID_NODE for a
+        deleted node) for rewriting the caller's NodeId map.  Without deletions: the identity map, nothing changes.  A
+        writer call, like insert and delete."""
+        o2n = np.zeros(max(self.n, 1), np.uint32)
+        n_new = C.c_uint64(0)
+        _check(_lib.load().turdb_cuda_index_compact(self._h, _ptr(o2n, C.c_uint32), C.byref(n_new)))
+        o2n = o2n[:self.n]
+        self.n = int(n_new.value)
+        return o2n
+
     def export_graph(self, with_vectors: bool = True) -> dict:
         """The graph the device holds, as the flat arrays from_graph takes (turdb_cuda_index_export_graph)."""
         L = _lib.load()
