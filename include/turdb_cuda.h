@@ -414,6 +414,33 @@ int32_t turdb_cuda_shards_search_batch(turdb_cuda_index* const* shards, uint32_t
                                        uint32_t ef, uint8_t metric, uint64_t* out_row_ids,
                                        float* out_dist, uint32_t* out_counts);
 
+/*
+ * ---- the SQL vector-scan operator over sub-indexes: ORDER BY vec <op> '[...]' LIMIT limit OFFSET offset -------------
+ * Table: the concatenation of the shards' live rows — shard 0's live rows in node-id order, then shard 1's, and so on
+ * (the contiguous row-range partition of tools/run_sharded.py).  Primary-key (scan) order is that concatenation.
+ *
+ * Result: for every statement exactly what turdb_cuda_sql_topk_batch(use_index = 0) returns on ONE index holding that
+ * concatenated table: row ids, f64 key bits, out_proj bits, counts, unused slots (TURDB_INVALID_ROW / NaN) and the
+ * order among equal keys.  Order among NULL keys is unspecified, as in the single form.  There is no index-backed form.
+ *
+ * Arguments: as turdb_cuda_sql_topk_batch (host pointers; out_* [nq][limit]; op 0 `<->`, 1 `<=>`, `<#>` is
+ * TURDB_ERR_UNSUPPORTED; proj_op 0..2 when out_proj is non-null; limit + offset <= TURDB_SQL_MAX_LIMIT_PLUS_OFFSET;
+ * limit 0 gives counts 0).  n_shards is 1..32; every shard has the query dimension and fewer than 2^31 nodes.  Shards
+ * may be on one device or on several; empty shards and shards whose rows are all deleted are allowed.  The operators
+ * and the window are checked first, then the shards; every check happens before any device work.
+ *
+ * How: every shard runs the certified filter of the exact scan over its own rows, all shards at once.  Then the
+ * reference's heap is relayed shard to shard in table order: shard s starts from the heap shard s - 1 left (copied
+ * device to device), replays its own candidates in scan order, or runs the reference's loop over its rows for a
+ * statement whose candidate buffers overflowed there, and hands the heap on; the last shard holding rows sorts and
+ * writes the window (DESIGN §8.1).  Concurrency: a READER call on every shard.
+ */
+int32_t turdb_cuda_shards_sql_topk_batch(turdb_cuda_index* const* shards, uint32_t n_shards,
+                                         const float* queries, uint32_t query_dim, uint32_t nq,
+                                         uint32_t limit, uint32_t offset, uint8_t op, uint8_t proj_op,
+                                         uint64_t* out_row_ids, double* out_keys, double* out_proj,
+                                         uint32_t* out_counts);
+
 /* The same merge over ONE packed block per shard — row ids [nq][k] u64 | distances [nq][k] f32 | counts [nq] u32 —,
  * blocks shard_stride_bytes apart (a multiple of 8): the output of a single all-gather of every rank's block. */
 int32_t turdb_cuda_merge_topk_packed_device(int32_t device, const void* d_gathered,

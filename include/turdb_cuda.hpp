@@ -254,4 +254,21 @@ class VectorTopKExec {
   std::vector<std::pair<uint64_t, double>> result_;
 };
 
+// turdb_cuda_shards_sql_topk_batch: nq statements `ORDER BY vec <op> literal LIMIT limit OFFSET offset` over the table
+// made of `shards`' live rows in shard order.  rows / keys are resized to [nq][limit], counts to [nq].
+inline void shards_sql_topk(const std::vector<const CudaHnswIndex*>& shards, const std::vector<float>& literals, uint32_t dim,
+                            VectorOp op, uint32_t limit, uint32_t offset, std::vector<uint64_t>& rows, std::vector<double>& keys,
+                            std::vector<uint32_t>& counts) {
+  std::vector<turdb_cuda_index*> handles;
+  for (const CudaHnswIndex* s : shards) handles.push_back(s->handle());
+  const uint32_t nq = dim ? (uint32_t)(literals.size() / dim) : 0;
+  rows.assign((size_t)nq * std::max<uint32_t>(limit, 1), TURDB_INVALID_ROW);
+  keys.assign(rows.size(), 0.0);
+  counts.assign(nq, 0);
+  check(turdb_cuda_shards_sql_topk_batch(handles.data(), (uint32_t)handles.size(), literals.data(), dim, nq, limit, offset,
+                                         (uint8_t)op, 0, rows.data(), keys.data(), nullptr, counts.data()));
+  rows.resize((size_t)nq * limit);
+  keys.resize((size_t)nq * limit);
+}
+
 }  // namespace turdb_cuda

@@ -57,6 +57,7 @@ EXPORTS = [
     "turdb_cuda_index_build", "turdb_cuda_index_export_graph", "turdb_cuda_index_insert",
     "turdb_cuda_sql_range_batch", "turdb_cuda_sql_range_batch_device", "turdb_cuda_sql_range_topk_batch",
     "turdb_cuda_sql_range_topk_batch_device", "turdb_cuda_index_delete", "turdb_cuda_index_compact",
+    "turdb_cuda_shards_sql_topk_batch",
 ]
 
 _lib = None
@@ -105,6 +106,8 @@ def load():
     L.turdb_cuda_index_enable_sq8.argtypes = [vp, pu8, u64, pu32]
     L.turdb_cuda_search_batch_sq8_device.argtypes = [vp, vp, u32, u32, u32, u32, u8, vp, vp, vp, vp, vp, vp, vp]
     L.turdb_cuda_shards_search_batch.argtypes = [C.POINTER(vp), u32, pf, u32, u32, u32, u32, u8, pu64, pf, pu32]
+    L.turdb_cuda_shards_sql_topk_batch.argtypes = [C.POINTER(vp), u32, pf, u32, u32, u32, u32, u8, u8, pu64,
+                                                    C.POINTER(C.c_double), C.POINTER(C.c_double), pu32]
     L.turdb_cuda_index_build.argtypes = [C.POINTER(BuildParams), u64, pf, pu64, C.POINTER(C.c_double), i32, C.POINTER(vp)]
     L.turdb_cuda_index_insert.argtypes = [vp, C.POINTER(BuildParams), u64, pf, pu64, C.POINTER(C.c_double)]
     L.turdb_cuda_index_delete.argtypes = [vp, u64, pu32, pu64]

@@ -1104,6 +1104,7 @@ extern "C" int32_t turdb_cuda_index_gather_probe(turdb_cuda_index* idx, uint32_t
 
 #include "sql_topk.inl"
 #include "sql_range.inl"
+#include "sql_shards.inl"
 #include "hnsw_file.inl"
 #include "graph_insert.inl"
 #include "graph_compact.inl"

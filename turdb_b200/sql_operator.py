@@ -12,6 +12,8 @@ BASELINE.json config 5's batch path).  All arithmetic is below the C ABI (csrc/s
 The distance-range scan `SELECT ... WHERE vec <op> '[...]' <cmp> r [LIMIT k [OFFSET o]]` (a Filter over the scan) runs
 through `VectorRangeScanBatch` (csrc/sql_range.inl), and both clauses together with one literal,
 `... WHERE vec <op> '[...]' < r ORDER BY vec <op> '[...]' LIMIT k` (TopK over the Filter), through `VectorRangeTopKBatch`.
+A table split into sub-indexes (one per GPU, or several on one) answers `ORDER BY ... LIMIT k` through
+`ShardedVectorScanBatch` (csrc/sql_shards.inl).
 """
 from __future__ import annotations
 
@@ -200,6 +202,62 @@ class VectorRangeTopKBatch:
                                                                   int(self.order_op), int(self.project or 0), self.limit,
                                                                   self.offset, d_rows or None, d_keys or None,
                                                                   d_proj or None, d_counts, stream or None))
+
+
+class ShardedVectorScanBatch:
+    """nq statements `SELECT [vec <project> literal_i] ... ORDER BY vec <op> literal_i LIMIT limit OFFSET offset` against
+    one table split into sub-indexes (csrc/sql_shards.inl): the table is shard 0's live rows in node-id order, then
+    shard 1's, and so on, and the result is row for row VectorScanBatch's (exact scan) on one index holding that
+    concatenation.  Raises ValueError before the library is called on an unknown or unsupported operator (`<#>` as the
+    sort key), limit + offset > SQL_MAX_LIMIT_PLUS_OFFSET, a shard list that is not 1..32 indexes of one dimension, or a
+    bad literal."""
+
+    def __init__(self, shards, op: VectorOp, limit: int, offset: int = 0, project: VectorOp | None = None):
+        try:
+            self.op = VectorOp(op)
+            self.project = None if project is None else VectorOp(project)
+        except ValueError as e:
+            raise ValueError(f"unknown operator: {e}") from None
+        if self.op == VectorOp.InnerProduct:
+            raise ValueError("ORDER BY <#> is NULL for every row in the reference; only <-> and <=> are sort keys")
+        limit, offset = int(limit), int(offset)
+        if not (0 <= limit < 2**32 and 0 <= offset < 2**32):
+            raise ValueError("limit and offset must be in [0, 2^32)")
+        if limit + offset > SQL_MAX_LIMIT_PLUS_OFFSET:
+            raise ValueError(f"limit + offset = {limit + offset} > {SQL_MAX_LIMIT_PLUS_OFFSET}")
+        self.shards = list(shards)
+        if not 1 <= len(self.shards) <= 32:
+            raise ValueError(f"need 1..32 shards, got {len(self.shards)}")
+        dims = {s.dim for s in self.shards}
+        if len(dims) != 1:
+            raise ValueError(f"shards of different dimensions: {sorted(dims)}")
+        self.dim = dims.pop()
+        self.limit, self.offset = limit, offset
+        self.projected = None
+
+    def execute(self, literals) -> tuple[np.ndarray, np.ndarray, np.ndarray]:
+        """-> (row_ids u64 [nq, limit], keys f64 [nq, limit] (NaN = NULL), counts u32 [nq]); unused slots are
+        INVALID_ROW / NaN.  The projected values, when asked for, are left in `self.projected` (f64 [nq, limit])."""
+        q = np.asarray(literals)
+        if q.ndim == 1:
+            q = q[None, :]
+        if q.dtype.kind != "f" or q.ndim != 2 or q.shape[1] != self.dim:
+            raise ValueError(f"literals must be float [nq, {self.dim}], got {q.dtype} {q.shape}")
+        q = np.ascontiguousarray(q, dtype=np.float32)
+        nq = q.shape[0]
+        lim = max(self.limit, 1)
+        rows = np.full((nq, lim), INVALID_ROW, np.uint64)
+        keys = np.full((nq, lim), np.nan, np.float64)
+        proj = np.full((nq, lim), np.nan, np.float64) if self.project is not None else None
+        counts = np.zeros(nq, np.uint32)
+        handles = (C.c_void_p * len(self.shards))(*[s._h for s in self.shards])
+        _check(_lib.load().turdb_cuda_shards_sql_topk_batch(handles, len(self.shards), _ptr(q, C.c_float), self.dim, nq,
+                                                            self.limit, self.offset, int(self.op), int(self.project or 0),
+                                                            _ptr(rows, C.c_uint64), _ptr(keys, C.c_double),
+                                                            _ptr(proj, C.c_double) if proj is not None else None,
+                                                            _ptr(counts, C.c_uint32)))
+        self.projected = None if proj is None else proj[:, :self.limit]
+        return rows[:, :self.limit], keys[:, :self.limit], counts
 
 
 class VectorTopKExec:
